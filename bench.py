@@ -282,7 +282,7 @@ def run_reference(args, rank: int, world: int):
     search, what = _cpu_search()
     threads = host_threads()
     rows, queries = 1_000_000, N_QUERIES
-    steps, warmup = max(args.steps, 1), max(args.warmup, 0)
+    steps, warmup = args.steps, max(args.warmup, 0)
     cat, qry = _cpu_sample(rows, queries)
     search(cat[: 1 << 17], qry[:64], TOPK, threads)   # start the thread pools
     t0 = time.perf_counter()
@@ -809,8 +809,7 @@ def run_serve_block(ctx: Ctx, steps: int, warmup: int):
                 q_op = index.prepare_queries(emb, normalize=False)
                 return sharded.search(q_op, K5)
 
-        n_steps = max(3, steps // 2) if Q < 1024 else steps
-        ms = timed(ctx, step, n_steps, max(warmup, 3))
+        ms = timed(ctx, step, steps, max(warmup, 3))
         n_local = hi - lo
         flops = 2.0 * Q * n_local * D5
         bytes_ = n_local * D5 * 2.0 + Q * D5 * 2 + Q * K5 * 12
@@ -888,7 +887,14 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="retrieval only (skip every extra block)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--blocks", default="train,ml1m,epoch,cfg4,serve", help="extra blocks to run (comma separated)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the top-K scores and ids of the last timed search as DIR/topk_scores.npy (float32) and "
+                         "DIR/topk_ids.npy (float64), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -909,7 +915,7 @@ def main():
         dist.init_process_group("nccl", device_id=device)
     ctx = Ctx(device, world, rank)
     warmup = max(args.warmup, 3)
-    steps = max(args.steps, 1)
+    steps = args.steps
     blocks = set() if args.no_train else {b for b in args.blocks.split(",") if b}
     want_cpu = (not args.no_cpu_baseline) and rank == 0 and world == 1
 
@@ -937,6 +943,11 @@ def main():
     ctx.barrier()
     ms = e0.elapsed_time(e1) / steps
     launches = N.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed search received in its last step (ids as float64: exact below 2^53)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "topk_scores.npy"), s.float().cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, "topk_ids.npy"), i.cpu().numpy().astype(np.float64))
     if rank == 0:
         sampler.rows = sampler.rows[n_before:] or sampler.rows[-3:]
     clocks = sampler.stop() if rank == 0 else None
@@ -954,7 +965,7 @@ def main():
     lib.b200rec_debug_topk_kernel_timing.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_float)]
     lib.b200rec_debug_topk_kernel_timing(1, None)
     kms = []
-    for _ in range(min(steps, 10)):
+    for _ in range(steps):
         sharded.search(q_op, TOPK)
         out = ctypes.c_float(0)
         lib.b200rec_debug_topk_kernel_timing(1, ctypes.byref(out))
@@ -990,32 +1001,31 @@ def main():
     e2e_same = bool(np.array_equal(i_np, np.asarray(i_sync)[lo_q:hi_q] if world > 1 else np.asarray(i_sync)))
     ctx.barrier()
     t0 = time.perf_counter()
-    for _ in range(max(3, steps // 2)):
+    for _ in range(steps):
         sync_call()
     ctx.barrier()
-    sync_ms = (time.perf_counter() - t0) / max(3, steps // 2) * 1e3
+    sync_ms = (time.perf_counter() - t0) / steps * 1e3
     ms, e2e_ms, kernel_ms, sync_ms = ctx.max_over_ranks(ms, e2e_ms, kernel_ms, sync_ms)
 
     del sharded, index, q_op, s, i
     torch.cuda.empty_cache()
     extra = {}
-    bsteps = min(max(steps, 10), 30)
 
     def block(key, fn, *a, **kw):
         run_block(extra, world, key, fn, *a, **kw)
 
     if "train" in blocks:
-        block("train", run_table_train_block, ctx, bsteps, warmup, want_cpu, name="config 2 (synthetic)", NU=1_000_000,
+        block("train", run_table_train_block, ctx, steps, warmup, want_cpu, name="config 2 (synthetic)", NU=1_000_000,
               NI=100_000, edim=64, hidden=[128, 64], E=64, sparse_tables=False, check_dp=True)
     if "ml1m" in blocks and rank == 0 and world == 1:
-        block("train_ml1m", run_ml1m_block, ctx, 200, 20, want_cpu)
+        block("train_ml1m", run_ml1m_block, ctx, steps, 20, want_cpu)
     if "epoch" in blocks and rank == 0 and world == 1:
         block("epoch_ml1m", run_epoch_block, ctx)
     if "cfg4" in blocks:
-        block("train_cfg4", run_table_train_block, ctx, bsteps, warmup, False, name="config 4 (synthetic)",
+        block("train_cfg4", run_table_train_block, ctx, steps, warmup, False, name="config 4 (synthetic)",
               NU=50_000_000, NI=5_000_000, edim=128, hidden=[256, 128], E=128, sparse_tables=True, check_dp=False)
     if "serve" in blocks:
-        block("serve", run_serve_block, ctx, bsteps, warmup)
+        block("serve", run_serve_block, ctx, steps, warmup)
     cpu = None
     if want_cpu:
         threads = host_threads()

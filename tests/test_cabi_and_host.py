@@ -175,95 +175,117 @@ def test_state_dict_layout_and_param_counts():
     assert final.user_tower.mlp[0].weight.shape == (256, 3)  # [out, in] Linear layout
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not mounted")
+def _golden_state(name, prefix):
+    """(keys in order, {key: array}) of the state dict stored under `prefix.` in tests/golden/<name>.npz."""
+    g = np.load(os.path.join(ROOT, "tests", "golden", name + ".npz"))
+    keys = [k[len(prefix) + 1:] for k in g.files if k.startswith(prefix + ".")]
+    return keys, {k: g[prefix + "." + k] for k in keys}
+
+
+def _assert_same_state(module, golden, prefix, skip=lambda k: False):
+    keys, want = _golden_state(golden, prefix)
+    sd = module.state_dict()
+    assert list(sd.keys()) == keys, (golden, prefix)
+    for k in keys:
+        if not skip(k):
+            assert np.array_equal(sd[k].detach().cpu().numpy(), want[k]), (golden, prefix, k)
+
+
+def _overwritten_after_init(k):
+    """Entries the golden generators change after construction (tests/golden/make_golden.py randomize_bn: BatchNorm
+    affine parameters and Linear biases from a separate generator; the stored running statistics are post-forward)."""
+    return not (k.endswith(".weight") and (k.startswith("embeddings.") or k.split(".")[1] in ("0", "4", "8")))
+
+
 def test_same_init_and_keys_as_the_imported_reference():
-    sys.path.insert(0, "/root/reference")
-    try:
-        from src.models.two_tower import create_two_tower_model as ref_create
-    finally:
-        sys.path.pop(0)
-    from b200rec.two_tower import create_two_tower_model
-    cfg = {"embedding_dim": 32, "temperature": 0.07,
-           "user_tower": {"input_dim": 7, "hidden_layers": [48, 32], "categorical_features": {"a": 12, "b": 300}},
-           "item_tower": {"input_dim": 9, "hidden_layers": [48, 32], "categorical_features": {"g": 40},
-                          "use_content_embedding": True}}
-    torch.manual_seed(123)
-    ref = ref_create(cfg)
-    torch.manual_seed(123)
-    ours = create_two_tower_model(cfg)
-    rsd, osd = ref.state_dict(), ours.state_dict()
-    assert list(rsd.keys()) == list(osd.keys())
-    for k in rsd:
-        assert torch.equal(rsd[k], osd[k]), k  # same RNG consumption order => identical initial weights
-    assert ours.temperature == ref.temperature
+    """Same RNG consumption order as the reference => identical initial weights: the reference's factory built towers
+    with categorical tables (cat_*.npz) and an ItemTower with the content branch (content_branch.npz) from a seed; the
+    same seed here gives the same state-dict keys, layouts and initial Linear weights / embedding tables, bit for bit."""
+    from b200rec.two_tower import ItemTower, create_two_tower_model
+    for act in ("relu", "gelu"):
+        cfg = {"embedding_dim": 32, "temperature": 0.1,
+               "user_tower": {"input_dim": 10, "hidden_layers": [64, 32], "dropout_rate": 0.0, "activation": act,
+                              "categorical_features": {"category": 10, "subcategory": 5}},
+               "item_tower": {"input_dim": 15, "hidden_layers": [64, 32], "dropout_rate": 0.0, "activation": act,
+                              "categorical_features": {"genre": 30, "studio": 200}, "use_content_embedding": False}}
+        torch.manual_seed(20)
+        ours = create_two_tower_model(cfg)
+        _assert_same_state(ours.user_tower, f"cat_{act}", "user", _overwritten_after_init)
+        _assert_same_state(ours.item_tower, f"cat_{act}", "item", _overwritten_after_init)
+        assert ours.temperature == 0.1
+    torch.manual_seed(41)
+    it = ItemTower(input_dim=12, embedding_dim=32, hidden_layers=[64, 48], dropout_rate=0.0, activation="relu",
+                   categorical_features={"genre": 20}, use_content_embedding=True, content_embedding_dim=64)
+    _assert_same_state(it, "content_branch", "sd", lambda k: k.startswith("mlp.") and k.split(".")[1] in ("2", "6"))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not mounted")
 def test_checkpoints_are_interchangeable_with_the_reference(tmp_path):
-    """save_model / load_model in both directions (reference two_tower.py:516-546): a checkpoint written by b200rec loads
-    into the reference model and vice versa — same file keys, same state-dict keys and layouts, biases, temperature."""
-    sys.path.insert(0, "/root/reference")
-    try:
-        from src.models.two_tower import create_two_tower_model as ref_create
-    finally:
-        sys.path.pop(0)
+    """save_model / load_model in both directions (reference two_tower.py:516-546): a checkpoint in the reference's
+    layout holding the reference's own initial state (trajectory_120.npz) loads into b200rec, and what b200rec writes
+    has that layout — the same file keys, state-dict keys and tensors, biases and temperature."""
     from b200rec.two_tower import create_two_tower_model
-    cfg = {"embedding_dim": 16, "temperature": 0.09,
-           "user_tower": {"input_dim": 5, "hidden_layers": [24, 16], "categorical_features": {"a": 12}},
-           "item_tower": {"input_dim": 6, "hidden_layers": [24, 16], "categorical_features": {"g": 40, "h": 3},
-                          "use_content_embedding": True}}
-    for writer_is_ours in (True, False):
-        torch.manual_seed(5 + writer_is_ours)
-        src = (create_two_tower_model if writer_is_ours else ref_create)(cfg)
-        with torch.no_grad():
-            src.user_bias.fill_(0.25)
-            src.item_bias.fill_(-0.5)
-            for m in src.modules():
-                if isinstance(m, torch.nn.BatchNorm1d):
-                    m.running_mean.normal_()
-                    m.running_var.uniform_(0.5, 2.0)
-        src.temperature = 0.123
-        path = str(tmp_path / f"ckpt_{writer_is_ours}.pth")
-        src.save_model(path)
-        ck = torch.load(path, map_location="cpu", weights_only=False)
-        assert sorted(ck.keys()) == ["item_bias", "item_tower_state", "temperature", "user_bias", "user_tower_state"]
-        torch.manual_seed(99)
-        dst = (ref_create if writer_is_ours else create_two_tower_model)(cfg)
-        dst.load_model(path)
-        a, b = src.state_dict(), dst.state_dict()
-        assert list(a.keys()) == list(b.keys())
-        for k in a:
-            assert torch.equal(a[k], b[k]), k
-        assert dst.temperature == 0.123
-        assert dst.user_bias.item() == 0.25 and dst.item_bias.item() == -0.5
+    keys, ref = _golden_state("trajectory_120", "sd")
+    tower = lambda t: {k[len(t) + 1:]: torch.from_numpy(ref[k].copy()) for k in keys if k.startswith(t + ".")}
+    cfg = {"embedding_dim": 64, "temperature": 0.05,
+           "user_tower": {"input_dim": 3, "hidden_layers": [128, 64]},
+           "item_tower": {"input_dim": 20, "hidden_layers": [128, 64], "use_content_embedding": False}}
+    path = str(tmp_path / "reference_layout.pth")
+    torch.save({"user_tower_state": tower("user_tower"), "item_tower_state": tower("item_tower"), "temperature": 0.123,
+                "user_bias": torch.nn.Parameter(torch.tensor([0.25])),
+                "item_bias": torch.nn.Parameter(torch.tensor([-0.5]))}, path)
+    torch.manual_seed(99)
+    ours = create_two_tower_model(cfg)
+    ours.load_model(path)
+    _assert_same_state(ours.user_tower, "trajectory_120", "sd.user_tower")
+    _assert_same_state(ours.item_tower, "trajectory_120", "sd.item_tower")
+    assert ours.temperature == 0.123
+    assert ours.user_bias.item() == 0.25 and ours.item_bias.item() == -0.5
+    path2 = str(tmp_path / "ours.pth")
+    ours.save_model(path2)
+    ck = torch.load(path2, map_location="cpu", weights_only=False)
+    assert sorted(ck.keys()) == ["item_bias", "item_tower_state", "temperature", "user_bias", "user_tower_state"]
+    for t in ("user_tower", "item_tower"):
+        want = tower(t)
+        assert list(ck[t + "_state"].keys()) == list(want.keys())
+        for k, v in want.items():
+            assert torch.equal(ck[t + "_state"][k], v), (t, k)
+    assert ck["temperature"] == 0.123 and ck["user_bias"].item() == 0.25 and ck["item_bias"].item() == -0.5
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not mounted")
-@pytest.mark.parametrize("config", [None, {}, {"embedding_dim": 64, "hidden_layers": [128, 64], "dropout_rate": 0.3,
-                                               "temperature": 0.1, "activation": "gelu"}])
-def test_training_factory_matches_the_reference(config):
-    """create_two_tower_model_for_training (reference src/training/utils.py:14-71): same defaults, same RNG consumption
-    (bit-identical initial weights), same temperature / dropout / activation wiring, same parameter count helper."""
-    sys.path.insert(0, "/root/reference")
-    try:
-        from src.training.utils import count_parameters as ref_count, create_two_tower_model_for_training as ref_create
-    finally:
-        sys.path.pop(0)
+# golden -> (seed, user_dim, item_dim, config) the reference's create_two_tower_model_for_training was called with
+# (tests/golden/make_golden.py, make_golden_round2.py)
+_FACTORY_GOLDENS = {
+    "trajectory_120": (77, 3, 20, {"embedding_dim": 64, "hidden_layers": [128, 64], "dropout_rate": 0.0,
+                                   "temperature": 0.05}),
+    "step_ml1m": (11, 3, 20, {"embedding_dim": 128, "hidden_layers": [256, 128], "dropout_rate": 0.0,
+                              "temperature": 0.05}),
+    "step_small": (12, 6, 9, {"embedding_dim": 64, "hidden_layers": [128, 64], "dropout_rate": 0.0, "temperature": 0.1}),
+}
+
+
+@pytest.mark.parametrize("golden", sorted(_FACTORY_GOLDENS))
+def test_training_factory_matches_the_reference(golden):
+    """create_two_tower_model_for_training (reference src/training/utils.py:14-71) against what the reference's factory
+    built from the same seed: same RNG consumption (bit-identical initial weights: the whole state dict where the
+    generator stored it untouched, the Linear weights otherwise), same keys, temperature and parameter count."""
     from b200rec.training_utils import count_parameters, create_two_tower_model_for_training
-    args = (3, 20) if config is None else (3, 20, config)
-    torch.manual_seed(7)
-    ref = ref_create(*args)
-    torch.manual_seed(7)
-    ours = create_two_tower_model_for_training(*args)
-    rsd, osd = ref.state_dict(), ours.state_dict()
-    assert list(rsd.keys()) == list(osd.keys())
-    for k in rsd:
-        assert torch.equal(rsd[k], osd[k]), k
-    assert ours.temperature == ref.temperature and count_parameters(ours) == ref_count(ref)
-    drops = lambda m: [x.p for x in m.modules() if isinstance(x, torch.nn.Dropout)]
-    assert drops(ours.user_tower) == drops(ref.user_tower) and drops(ours.item_tower) == drops(ref.item_tower)
-    kinds = lambda m: [type(x).__name__ for x in m.mlp]
-    assert kinds(ours.user_tower) == kinds(ref.user_tower) and kinds(ours.item_tower) == kinds(ref.item_tower)
+    seed, ud, idim, cfg = _FACTORY_GOLDENS[golden]
+    torch.manual_seed(seed)
+    ours = create_two_tower_model_for_training(ud, idim, cfg)
+    if golden == "trajectory_120":
+        _assert_same_state(ours, golden, "sd")
+        user = _golden_state(golden, "sd.user_tower")[1]
+        item = _golden_state(golden, "sd.item_tower")[1]
+        temperature = cfg["temperature"]
+    else:
+        _assert_same_state(ours.user_tower, golden, "user", _overwritten_after_init)
+        _assert_same_state(ours.item_tower, golden, "item", _overwritten_after_init)
+        user, item = _golden_state(golden, "user")[1], _golden_state(golden, "item")[1]
+        temperature = float(np.load(os.path.join(ROOT, "tests", "golden", golden + ".npz"))["temperature"])
+    assert np.float32(ours.temperature) == np.float32(temperature)
+    learnable = sum(v.size for t in (user, item) for k, v in t.items() if "running" not in k and "num_batches" not in k)
+    assert count_parameters(ours) == learnable + 2      # + user_bias, item_bias
+    assert [x.p for x in ours.modules() if isinstance(x, torch.nn.Dropout)] == [cfg["dropout_rate"]] * 4
 
 
 def test_shard_bounds_cover_the_catalogue():

@@ -404,7 +404,13 @@ def test_oracle_content_projection_branch_matches_reference(golden_dir):
                 assert np.abs(grads[k] - ref).max() <= 2e-5 * max(np.abs(ref).max(), 1e-6), k
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not mounted")
+# a checkout of the original project (the reference the goldens were generated from), e.g. REFERENCE_ROOT=../upstream
+REFERENCE_ROOT = os.environ.get("REFERENCE_ROOT", "")
+needs_reference = pytest.mark.skipif(not (REFERENCE_ROOT and os.path.isdir(os.path.join(REFERENCE_ROOT, "src"))),
+                                     reason="set REFERENCE_ROOT to a checkout of the original project")
+
+
+@needs_reference
 def test_committed_goldens_regenerate_from_the_imported_reference(tmp_path):
     """Provenance of tests/golden/*.npz: every generator script is re-run here (each imports the unmodified reference and
     runs it on seeded inputs) and what it writes must equal the committed fixture — identical integer / string arrays,
@@ -421,7 +427,7 @@ def test_committed_goldens_regenerate_from_the_imported_reference(tmp_path):
     assert not problems, problems[:10]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference tree not mounted")
+@needs_reference
 @pytest.mark.parametrize("seed", range(6))
 def test_oracle_matches_the_live_reference_on_random_configurations(seed):
     """Beyond the stored fixtures: the numpy restatement against the IMPORTED reference itself (torch-CPU autograd) on
@@ -431,8 +437,8 @@ def test_oracle_matches_the_live_reference_on_random_configurations(seed):
     gradient (tables included) and the BatchNorm running statistics after the step."""
     import sys
     import torch
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
+    if REFERENCE_ROOT not in sys.path:
+        sys.path.insert(0, REFERENCE_ROOT)
     from src.models.two_tower import ItemTower, TwoTowerModel, UserTower
     rng = np.random.default_rng(1000 + seed)
     torch.manual_seed(1000 + seed)
