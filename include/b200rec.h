@@ -67,6 +67,23 @@ int b200rec_flat_ip_topk(const void* catalogue, int64_t N, int64_t ld, const voi
                          int64_t row_offset, const int64_t* exclude_indptr, const int32_t* exclude_rows,
                          const float* tau_init, float* out_scores, int64_t* out_ids, void* workspace,
                          size_t workspace_bytes, void* stream);
+/* Filtered search: the exact top-k over the rows allowed by a row filter.  allow_bits is a bitmap over LOCAL rows in
+ * faiss' IDSelectorBitmap layout (bit r = bit r&7 of byte r>>3, LSB first; equivalently bit r&31 of little-endian
+ * uint32 word r>>5), allow_n its length in rows: rows >= allow_n are not allowed.  Same order, padding, workspace and
+ * limits as b200rec_flat_ip_topk; disallowed rows are rejected where candidates enter the running lists, and the
+ * internal sampling pass counts them as -inf.  Cost grows as the filter gets more selective (disallowed rows above the
+ * running threshold still take the slow path): for selective filters search a compacted catalogue instead
+ * (b200rec_gather_rows + b200rec_flat_ip_topk + b200rec_remap_ids). */
+int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
+                                  int64_t row_offset, const uint32_t* allow_bits, int64_t allow_n, float* out_scores,
+                                  int64_t* out_ids, void* workspace, size_t workspace_bytes, void* stream);
+/* Row filters (csrc/filter.cu).  bits [ceil(n_bits/32)] uint32 = the bitmap of the rows[0..n) that lie in [0, n_bits)
+ * (out-of-range rows are ignored, duplicates are harmless; the bitmap is cleared first; rows may be NULL when n = 0).  b200rec_remap_ids maps the
+ * ids of a search over a compacted catalogue (row j = catalogue row rows[j], rows ascending) back:
+ * out[i] = rows[ids[i]] + row_offset, -1 stays -1 (in place allowed). */
+int b200rec_rows_to_bitmap(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, void* stream);
+int b200rec_remap_ids(const int64_t* ids, int64_t n, const int64_t* rows, int64_t n_rows, int64_t row_offset,
+                      int64_t* out, void* stream);
 /* Sampling pass alone: out_vals [Q,k_out] = the k_out (<= k) largest group maxima (distinct sampled rows) of every
  * query, descending.  Row-sharded search exchanges these (all-gather) and starts every shard from the k-th best of the
  * union; `shards` (>= 1) says how many shards pool their samples, so each one samples 1/shards as densely.

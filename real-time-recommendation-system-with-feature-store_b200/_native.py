@@ -30,6 +30,9 @@ SIGNATURES = {
     "b200rec_gemm_bf16_tn": (_I, [_P, _I64, _I64, _P, _I64, _I64, _I64, _P, _I64, _P, _F, _I, _P]),
     "b200rec_topk_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I]),
     "b200rec_flat_ip_topk": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "b200rec_flat_ip_topk_filtered": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _I64, _P, _P, _P, _SZ, _P]),
+    "b200rec_rows_to_bitmap": (_I, [_P, _I64, _I64, _P, _P]),
+    "b200rec_remap_ids": (_I, [_P, _I64, _P, _I64, _I64, _P, _P]),
     "b200rec_topk_sample": (_I, [_P, _I64, _I64, _P, _I64, _I, _I, _I, _P, _P, _SZ, _P]),
     "b200rec_topk_has_sample": (_I, [_I64, _I64, _I64, _I]),
     "b200rec_topk_pooled_kth": (_I, [_P, _I, _I64, _I, _I, _P, _P]),

@@ -100,6 +100,11 @@ __device__ __forceinline__ void warp_select_threshold(const Loader& load, int n,
   shift_out = shift;
 }
 
+// row filter: bit r of the bitmap (LSB first, faiss IDSelectorBitmap layout); rows past allow_n are not allowed
+__device__ __forceinline__ bool row_allowed(const uint32_t* bits, uint32_t n, uint32_t row) {
+  return row < n && ((__ldg(bits + (row >> 5)) >> (row & 31u)) & 1u) != 0u;
+}
+
 __device__ __noinline__ bool row_excluded(const int32_t* rows, int n, uint32_t row) {
   int lo = 0, hi = n;
   while (lo < hi) {
@@ -140,6 +145,8 @@ struct TopkArgs {
   uint32_t* left;                 // [grid][128*NQ]  leftover (list id << 31 | count) of each CTA's last segment
   const int64_t* excl_indptr;     // [Q+1] or null
   const int32_t* excl_rows;       // sorted per query
+  const uint32_t* allow;          // row filter bitmap (bit r = bit r&31 of word r>>5) or null; rows >= allow_n are out
+  uint32_t allow_n;
   int k;
   int cap;
   int flush;  // hand a list to the helper warps once it holds this many candidates (keeps tau fresh)
@@ -247,7 +254,7 @@ struct TopkEpiT {
   // instruction cache and free of branches (a fully unrolled 64-column scan with an inlined exclusion search was
   // 70 KB of SASS and spent 80% of its issue slots waiting for instruction fetch).
   __device__ __forceinline__ void append(const Args& ea, int a, float x, uint32_t row) {
-    if (ex_n[a] == 0 || !row_excluded(ex_lo[a], ex_n[a], row)) {
+    if ((ex_n[a] == 0 || !row_excluded(ex_lo[a], ex_n[a], row)) && (ea.allow == nullptr || row_allowed(ea.allow, ea.allow_n, row))) {
       __stcg(buf[a] + (active[a] ? ea.cap : 0) + cnt[a], make_key(x, row));
       ++cnt[a];
       if (dbgv(ea) == 2) ++n_app;
@@ -641,15 +648,23 @@ using TopkEpiDbg = TopkEpiT<true>;
 // maxima belong to distinct rows, so the k-th largest of them is a valid lower bound of the final k-th score; with
 // thousands of groups per query it is nearly as tight as the exact k-th of the whole sample, and it costs no
 // selection at all.  It removes the cold-start phase in which almost every score is a candidate.
+// MASK = true (filtered search): sampled rows outside the row filter count as -inf, so the group maxima stay a lower
+// bound of the k-th ALLOWED score; a threshold taken from disallowed rows could exceed it and drop results.
 // ---------------------------------------------------------------------------------------------------------------
-struct SampleMaxEpi {
+struct SampleArgs {
+  float* out;              // [Q][ngroups]
+  int ngroups;             // m / gw
+  int gw;                  // 32, 64 or 128 sampled rows per group
+  const uint32_t* allow;   // MASK only: row filter bitmap and its length in rows
+  uint32_t allow_n;
+  uint32_t stride;         // MASK only: sampled row j is catalogue row j * stride
+};
+
+template <bool MASK>
+struct SampleMaxEpiT {
   static constexpr bool kDbg = false;
   static constexpr int SCRATCH_BYTES = 64;
-  struct Args {
-    float* out;     // [Q][ngroups]
-    int ngroups;    // m / gw
-    int gw;         // 32, 64 or 128 sampled rows per group
-  };
+  using Args = SampleArgs;
   long long qrow[2];
 
   static __device__ __forceinline__ void init_scratch(uint32_t*, int) {}
@@ -675,6 +690,12 @@ struct SampleMaxEpi {
       uint32_t v[32];
       tmem_ld_32x32(taddr + c, v);
       tmem_ld_wait();
+      if (MASK) {  // column c + i of the tile is sampled row row0 + c + i: one bitmap probe per lane, one vote
+        const unsigned long long row = (row0 + c + (threadIdx.x & 31u)) * (unsigned long long)ea.stride;
+        const uint32_t ok = __ballot_sync(FULL_MASK, row < ea.allow_n && row_allowed(ea.allow, ea.allow_n, (uint32_t)row));
+#pragma unroll
+        for (int i = 0; i < 32; ++i) v[i] = ((ok >> i) & 1u) ? v[i] : __float_as_uint(-INFINITY);
+      }
       float m4[4];
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
@@ -694,6 +715,7 @@ struct SampleMaxEpi {
   __device__ __forceinline__ void end_segment(const Args&, const StreamGeom&, int, int, const int (&)[QPT], int,
                                               uint32_t*, bool) {}
 };
+using SampleMaxEpi = SampleMaxEpiT<false>;
 
 // ---------------------------------------------------------------------------------------------------------------
 // block-level exact select + sort of `n` keys produced by a loader; one CTA (256 threads) per query
@@ -1242,8 +1264,8 @@ static int plan_topk(TopkPlan& p, int64_t N, int64_t ld, int64_t Q, int k, int s
 template <int NQ, int BN, int V2, bool DBG>
 static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
                        int k, int64_t row_offset, const int64_t* excl_indptr, const int32_t* excl_rows,
-                       float* out_scores, int64_t* out_ids, void* workspace, cudaStream_t st,
-                       const float* tau_init, float* sample_vals_out, const OutFan* fan_in) {
+                       const uint32_t* allow, int64_t allow_n, float* out_scores, int64_t* out_ids, void* workspace,
+                       cudaStream_t st, const float* tau_init, float* sample_vals_out, const OutFan* fan_in) {
   OutFan fan;
   if (fan_in != nullptr) {
     fan = *fan_in;
@@ -1266,6 +1288,8 @@ static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int6
   B200_CUDA_OK(cudaMemsetAsync(ea.left, 0, p.left_bytes, st));
   ea.excl_indptr = excl_indptr;
   ea.excl_rows = excl_rows;
+  ea.allow = allow;
+  ea.allow_n = (uint32_t)allow_n;
   ea.k = k;
   ea.cap = p.cap;
   // hand a list over every ~k/4 candidates: each merge selects over k + list keys, so the threshold scales with k
@@ -1291,17 +1315,23 @@ static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int6
     float* S = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(workspace) + p.lists_bytes + p.tlists_bytes + p.meta_bytes + p.left_bytes);
     CUtensorMap ts;  // row i of this map is catalogue row i * stride
     if (cached_tmap(&ts, catalogue, (uint64_t)p.sample_m, (uint64_t)ld, (uint64_t)(ld * p.sample_stride), XBOX)) return 1;
-    SampleMaxEpi::Args sa;
+    SampleArgs sa;
     sa.out = S;
     sa.ngroups = (int)(p.sample_m / p.sample_gw);
     sa.gw = p.sample_gw;
-    void (*skern)(const CUtensorMap, const CUtensorMap, const StreamGeom, const SampleMaxEpi::Args);
-    if constexpr (V2 != 0) skern = stream_scores2_kernel<(V2 == 2 ? 2 : 1), SampleMaxEpi>;
-    else skern = stream_scores_kernel<NQ, BN, SampleMaxEpi>;
-    static bool sattr = false;
-    if (!sattr) {
+    sa.allow = allow;
+    sa.allow_n = (uint32_t)allow_n;
+    sa.stride = (uint32_t)p.sample_stride;
+    void (*skern)(const CUtensorMap, const CUtensorMap, const StreamGeom, const SampleArgs);
+    if constexpr (V2 != 0) {
+      skern = allow ? stream_scores2_kernel<(V2 == 2 ? 2 : 1), SampleMaxEpiT<true>> : stream_scores2_kernel<(V2 == 2 ? 2 : 1), SampleMaxEpi>;
+    } else {
+      skern = allow ? stream_scores_kernel<NQ, BN, SampleMaxEpiT<true>> : stream_scores_kernel<NQ, BN, SampleMaxEpi>;
+    }
+    static bool sattr[2] = {false, false};
+    if (!sattr[allow ? 1 : 0]) {
       B200_CUDA_OK(cudaFuncSetAttribute(skern, cudaFuncAttributeMaxDynamicSharedMemorySize, ST_SMEM_LIMIT));
-      sattr = true;
+      sattr[allow ? 1 : 0] = true;
     }
     skern<<<p.gs.grid, ST_THREADS, p.gs.smem_bytes, st>>>(tq, ts, p.gs, sa);
     B200_LAUNCH_OK("stream_scores_kernel<sample>");
@@ -1409,7 +1439,8 @@ extern "C" size_t b200rec_topk_workspace_bytes(int64_t N, int64_t ld, int64_t Q,
 
 static int topk_dispatch(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
                          int64_t row_offset, const int64_t* exclude_indptr, const int32_t* exclude_rows,
-                         const float* tau_init, float* out_scores, int64_t* out_ids, float* sample_vals_out,
+                         const uint32_t* allow, int64_t allow_n, const float* tau_init, float* out_scores,
+                         int64_t* out_ids, float* sample_vals_out,
                          int sample_k_out, int shards, const b200::OutFan* fan,
                          void* workspace, size_t workspace_bytes, void* stream) {
   using namespace b200;
@@ -1421,7 +1452,7 @@ static int topk_dispatch(const void* catalogue, int64_t N, int64_t ld, const voi
   if ((exclude_indptr == nullptr) != (exclude_rows == nullptr)) return fail("topk: exclusion CSR needs both arrays");
   if (sample_vals_out != nullptr && p.sample_m == 0) return fail("topk_sample: catalogue too small for a sampling pass");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-#define B200_TOPK_ARGS p, catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, out_scores, out_ids, workspace, st, tau_init, sample_vals_out, fan
+#define B200_TOPK_ARGS p, catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, allow, allow_n, out_scores, out_ids, workspace, st, tau_init, sample_vals_out, fan
   if (knobs().debug != 0 || knobs().stream_stats || knobs().stats_unit >= 0) {  // development instantiation
     if (p.v2 == 2) return launch_topk<2, 128, 2, true>(B200_TOPK_ARGS);
     if (p.v2 == 1) return launch_topk<2, 128, 1, true>(B200_TOPK_ARGS);
@@ -1442,8 +1473,19 @@ extern "C" int b200rec_flat_ip_topk(const void* catalogue, int64_t N, int64_t ld
                                     const float* tau_init, float* out_scores, int64_t* out_ids, void* workspace,
                                     size_t workspace_bytes, void* stream) {
   if (!catalogue || !queries || !out_scores || !out_ids || !workspace) return b200::fail("topk: null pointer");
-  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, tau_init, out_scores,
-                       out_ids, nullptr, k, 1, nullptr, workspace, workspace_bytes, stream);
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, nullptr, 0, tau_init,
+                       out_scores, out_ids, nullptr, k, 1, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                             int k, int64_t row_offset, const uint32_t* allow_bits, int64_t allow_n,
+                                             float* out_scores, int64_t* out_ids, void* workspace,
+                                             size_t workspace_bytes, void* stream) {
+  if (!catalogue || !queries || !allow_bits || !out_scores || !out_ids || !workspace)
+    return b200::fail("topk_filtered: null pointer");
+  if (allow_n < 0) return b200::fail("topk_filtered: allow_n must be >= 0");
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, allow_bits, allow_n < N ? allow_n : N,
+                       nullptr, out_scores, out_ids, nullptr, k, 1, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int b200rec_topk_sample(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
@@ -1451,7 +1493,7 @@ extern "C" int b200rec_topk_sample(const void* catalogue, int64_t N, int64_t ld,
                                    void* stream) {
   if (!catalogue || !queries || !out_vals || !workspace) return b200::fail("topk_sample: null pointer");
   if (k_out < 1 || k_out > k) return b200::fail("topk_sample: k_out must be in [1, k]");
-  return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, nullptr, nullptr, out_vals, k_out,
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, out_vals, k_out,
                        shards < 1 ? 1 : shards, nullptr, workspace, workspace_bytes, stream);
 }
 
@@ -1474,7 +1516,7 @@ extern "C" int b200rec_flat_ip_topk_fanout(const void* catalogue, int64_t N, int
   if (!catalogue || !queries || !workspace) return b200::fail("topk: null pointer");
   b200::OutFan fan;
   if (make_fan(fan, n_dst, dst_scores, dst_ids, true)) return 1;
-  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, tau_init, fan.s[0], fan.i[0], nullptr, k,
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, nullptr, 0, tau_init, fan.s[0], fan.i[0], nullptr, k,
                        1, &fan, workspace, workspace_bytes, stream);
 }
 
@@ -1485,7 +1527,7 @@ extern "C" int b200rec_topk_sample_fanout(const void* catalogue, int64_t N, int6
   if (k_out < 1 || k_out > k) return b200::fail("topk_sample: k_out must be in [1, k]");
   b200::OutFan fan;
   if (make_fan(fan, n_dst, dst_vals, nullptr, false)) return 1;
-  return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, nullptr, nullptr, fan.s[0], k_out,
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, fan.s[0], k_out,
                        shards < 1 ? 1 : shards, &fan, workspace, workspace_bytes, stream);
 }
 

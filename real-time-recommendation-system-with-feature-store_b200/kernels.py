@@ -105,6 +105,44 @@ def flat_ip_topk(catalogue: torch.Tensor, queries: torch.Tensor, k: int, row_off
     return scores, ids
 
 
+def flat_ip_topk_filtered(catalogue: torch.Tensor, queries: torch.Tensor, k: int, allow_bits: torch.Tensor,
+                          allow_n: int, row_offset: int = 0, workspace: Optional[torch.Tensor] = None
+                          ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """flat_ip_topk over the rows allowed by a bitmap (int32/uint32 words, bit r of word r >> 5; rows >= allow_n out)."""
+    assert catalogue.dtype == BF16 and queries.dtype == BF16 and allow_bits.dtype == torch.int32
+    assert catalogue.stride(1) == 1 and queries.stride(1) == 1 and catalogue.stride(0) == queries.stride(0)
+    n, ld = catalogue.shape[0], catalogue.stride(0)
+    q = queries.shape[0]
+    assert allow_bits.numel() * 32 >= min(allow_n, n)
+    need = topk_workspace_bytes(n, ld, q, k)
+    if need == 0:
+        raise RuntimeError(f"b200rec flat_ip_topk_filtered: {N.last_error()}")
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty((need,), dtype=torch.uint8, device=catalogue.device)
+    scores = torch.empty((q, k), dtype=torch.float32, device=catalogue.device)
+    ids = torch.empty((q, k), dtype=torch.int64, device=catalogue.device)
+    N.check(N.lib().b200rec_flat_ip_topk_filtered(N.ptr(catalogue), n, ld, N.ptr(queries), q, k, row_offset,
+                                                  N.ptr(allow_bits), allow_n, N.ptr(scores), N.ptr(ids),
+                                                  N.ptr(workspace), workspace.numel(), N.stream()), "flat_ip_topk_filtered")
+    return scores, ids
+
+
+def rows_to_bitmap(rows: torch.Tensor, n_bits: int) -> torch.Tensor:
+    """int64 rows -> int32 [ceil(n_bits / 32)] bitmap (faiss IDSelectorBitmap layout); rows outside [0, n_bits) ignored."""
+    assert rows.dtype == torch.int64 and rows.is_contiguous()
+    bits = torch.empty(((n_bits + 31) // 32,), dtype=torch.int32, device=rows.device)
+    N.check(N.lib().b200rec_rows_to_bitmap(N.ptr(rows), rows.numel(), n_bits, N.ptr(bits), N.stream()), "rows_to_bitmap")
+    return bits
+
+
+def remap_ids(ids: torch.Tensor, rows: torch.Tensor, row_offset: int = 0) -> torch.Tensor:
+    """ids of a search over catalogue rows `rows` (ascending) -> rows[ids] + row_offset, in place; -1 stays -1."""
+    assert ids.dtype == torch.int64 and ids.is_contiguous() and rows.dtype == torch.int64 and rows.is_contiguous()
+    N.check(N.lib().b200rec_remap_ids(N.ptr(ids), ids.numel(), N.ptr(rows), rows.numel(), row_offset, N.ptr(ids),
+                                      N.stream()), "remap_ids")
+    return ids
+
+
 def topk_pooled_kth(vals: torch.Tensor, k: int) -> torch.Tensor:
     """vals [parts, Q, k_in] fp32 (contiguous) -> [Q]: k-th largest of each query's parts*k_in pooled sample maxima."""
     assert vals.dim() == 3 and vals.is_contiguous() and vals.dtype == torch.float32

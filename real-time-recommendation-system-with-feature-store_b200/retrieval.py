@@ -50,6 +50,41 @@ class IndexBase(ABC):
         pass
 
 
+class RowFilter:
+    """A fixed set of LOCAL rows of one `FlatIPDeviceIndex` (faiss' IDSelectorBatch semantics): built by
+    `FlatIPDeviceIndex.row_filter`, passed as `sel=` to `search_device` / `search`, which then return the exact top-k
+    over these rows only.  Rows added to the index after the filter was built are not allowed.
+
+    `rows` (int64, ascending, on the device) and `bits` (the IDSelectorBitmap of those rows, int32 words) are built once.
+    `compacted()` is the catalogue operand restricted to the allowed rows ([n_allowed, ld] bf16, n_allowed * ld * 2
+    bytes: 2.56 GB for an all-allowed filter over 10 M x 128 rows), gathered on first use and kept with the filter, so a
+    filter reused across requests ("in stock") pays the gather once; flat-index rows never move, so `add` does not
+    invalidate it."""
+
+    def __init__(self, index: "FlatIPDeviceIndex", rows: np.ndarray):
+        self.index = index
+        self.n_bits = index.ntotal
+        self.n_allowed = int(rows.size)
+        self.rows = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.int64)).to(index.device)
+        self.bits = K.rows_to_bitmap(self.rows, max(self.n_bits, 1))
+        self._compact: Optional[torch.Tensor] = None
+
+    @property
+    def fraction(self) -> float:
+        """Allowed share of the rows the index held when the filter was built."""
+        return self.n_allowed / max(self.n_bits, 1)
+
+    def compacted(self) -> torch.Tensor:
+        if self._compact is None:
+            ix = self.index
+            out = torch.empty((self.n_allowed, ix.ld), dtype=torch.bfloat16, device=ix.device)
+            err = torch.zeros((1,), dtype=torch.int32, device=ix.device)
+            # bf16 rows viewed as fp32 words (ld * 2 bytes is a multiple of 128 B): the feed's row gather does the copy
+            K.gather_rows(ix._cat[: self.n_bits].view(torch.float32), self.rows, err, out=out.view(torch.float32))
+            self._compact = out
+        return self._compact
+
+
 class FlatIPDeviceIndex:
     """faiss.IndexFlatIP on one B200: rows appended with `add`, exact `search`.
 
@@ -66,6 +101,12 @@ class FlatIPDeviceIndex:
         """Extra candidates the tensor-core pass hands to the exact fp32 re-scoring: enough that the true top-k are
         inside unless more than this many rows lie within the 3-product error of the k-th score."""
         return max(16, k // 4)
+
+    # Filtered search over a compacted copy of the allowed rows below this allowed fraction, with the row bitmap tested
+    # inside the fused kernel above it.  Measured on config 3 (DESIGN.md section 4, tools/filtered_search.py): the
+    # cached compact search is faster at every fraction, and at f <= 0.5 by 1.6-44x; at f = 1 it gains 8-13 % for a
+    # second 2.56 GB copy of the catalogue and a 1.8-2.0 ms first gather, so near-complete filters keep the bitmap.
+    FILTER_COMPACT_BELOW = 0.75
 
     def __init__(self, d: int, storage: str = "fp32", device: Optional[torch.device] = None, row_offset: int = 0):
         if storage not in ("bf16", "fp32"):
@@ -149,8 +190,8 @@ class FlatIPDeviceIndex:
             qop._b200_f32 = y if normalize else qt       # the fp32 queries travel with their operand (exact re-scoring)
         return qop
 
-    def _workspace(self, nq: int, k: int) -> torch.Tensor:
-        need = K.topk_workspace_bytes(self.ntotal, self.ld, nq, k)
+    def _workspace(self, nq: int, k: int, n: Optional[int] = None) -> torch.Tensor:
+        need = K.topk_workspace_bytes(self.ntotal if n is None else n, self.ld, nq, k)
         if need == 0:
             raise RuntimeError(f"b200rec flat_ip_topk: {K.N.last_error()}")
         if self._ws is None or self._ws.numel() < need:
@@ -173,10 +214,42 @@ class FlatIPDeviceIndex:
         K.flat_ip_topk_fanout(self._cat[: self.ntotal], q_op, k, self.row_offset, tau_init, dst_scores, dst_ids,
                               self._workspace(q_op.shape[0], k))
 
+    def row_filter(self, rows=None, mask=None) -> RowFilter:
+        """Row filter over the rows held now: `rows` (int array, numpy or torch; out-of-range and duplicate rows are
+        ignored) or `mask` (bool array of length <= ntotal; missing tail = not allowed)."""
+        if (rows is None) == (mask is None):
+            raise ValueError("row_filter takes exactly one of rows= or mask=")
+        if mask is not None:
+            m = np.asarray(mask.cpu() if torch.is_tensor(mask) else mask)
+            if m.dtype != np.bool_ or m.ndim != 1 or m.size > self.ntotal:
+                raise ValueError(f"mask must be a 1-D bool array of length <= ntotal ({self.ntotal})")
+            r = np.flatnonzero(m)
+        else:
+            r = np.asarray(rows.cpu() if torch.is_tensor(rows) else rows).reshape(-1)
+            if r.size and not np.issubdtype(r.dtype, np.integer):
+                raise ValueError("rows must be an integer array")
+            r = r.astype(np.int64, copy=False)
+            r = np.unique(r[(r >= 0) & (r < self.ntotal)])
+        return RowFilter(self, r)
+
     def search_device(self, q_op: torch.Tensor, k: int, exclude_indptr=None, exclude_rows=None, tau_init=None,
-                      out=None):
-        """q_op: bf16 operand [nq, ld] on the device -> (D, I) device tensors (written into `out` when given)."""
+                      out=None, sel: Optional[RowFilter] = None):
+        """q_op: bf16 operand [nq, ld] on the device -> (D, I) device tensors (written into `out` when given).
+        `sel` (a RowFilter of this index): exact top-k over the allowed rows only, -1 / -FLT_MAX padding past them."""
         nq = q_op.shape[0]
+        if sel is not None:
+            if exclude_indptr is not None or exclude_rows is not None:
+                raise ValueError("a row filter cannot be combined with per-query exclusion lists")
+            if tau_init is not None:
+                raise ValueError("a row filter cannot be combined with tau_init (row-sharded search)")
+            if sel.index is not self:
+                raise ValueError("the row filter was built for another index")
+            d, i = self._search_filtered(q_op, k, sel, sel.fraction < self.FILTER_COMPACT_BELOW)
+            if out is not None:
+                out[0].copy_(d)
+                out[1].copy_(i)
+                return out
+            return d, i
         if self.ntotal == 0:
             if out is not None:
                 out[0].fill_(-FLT_MAX)
@@ -199,11 +272,34 @@ class FlatIPDeviceIndex:
             return out
         return d, i
 
-    def search(self, q, k: int, normalize: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+    def _search_filtered(self, q_op: torch.Tensor, k: int, sel: RowFilter, compact: bool):
+        """Both exact filtered paths: compact = search the gathered allowed rows and map the ids back through the row
+        list; else the full catalogue with the row bitmap tested inside the fused kernel.  fp32 storage: k + margin
+        candidates among the allowed rows, re-scored from the fp32 rows as in search_device."""
+        nq = q_op.shape[0]
+        q32 = getattr(q_op, "_b200_f32", None) if self._f32 is not None else None
+        if compact and sel.n_allowed == 0:
+            return (torch.full((nq, k), -FLT_MAX, dtype=torch.float32, device=self.device),
+                    torch.full((nq, k), -1, dtype=torch.int64, device=self.device))
+        kk = k if q32 is None else min(k + self.rescore_margin(k), max(k, min(self.ntotal, 2048)))
+        if compact:
+            cat = sel.compacted()
+            d, i = K.flat_ip_topk(cat, q_op, kk, 0, workspace=self._workspace(nq, kk, cat.shape[0]))
+            K.remap_ids(i, sel.rows, self.row_offset)
+        else:
+            d, i = K.flat_ip_topk_filtered(self._cat[: self.ntotal], q_op, kk, sel.bits, sel.n_bits, self.row_offset,
+                                           self._workspace(nq, kk))
+        if q32 is None:
+            return d, i
+        exact = K.rescore_fp32(q32, self._f32[: self.ntotal], i, self.row_offset)
+        return K.topk_merge(exact.unsqueeze(0), i.unsqueeze(0), k)
+
+    def search(self, q, k: int, normalize: bool = False, sel: Optional[RowFilter] = None) -> Tuple[np.ndarray, np.ndarray]:
         """faiss contract: (D float32 [nq,k] descending, I int64 [nq,k]) as numpy arrays — `index.search(q, k)` of
-        reference retrieval.py:171.  Host queries travel through pinned staging buffers kept by the index."""
-        if torch.is_tensor(q) and q.is_cuda:
-            d, i = self.search_device(self.prepare_queries(q, normalize), k)
+        reference retrieval.py:171.  Host queries travel through pinned staging buffers kept by the index; a filtered
+        search (`sel`, see search_device) takes the blocking path."""
+        if sel is not None or (torch.is_tensor(q) and q.is_cuda):
+            d, i = self.search_device(self.prepare_queries(q, normalize), k, sel=sel)
             return d.cpu().numpy(), i.cpu().numpy()
         for out in self.search_stream([q], k, normalize):
             return out
@@ -310,6 +406,10 @@ class B200FlatIndex(IndexBase):
         self.nprobe = self.config.get("nprobe", 20)
         self.use_gpu = True
         self.storage = self.config.get("storage", "fp32")
+        self.filter = self.config.get("filter", "post")
+        if self.filter not in ("post", "exact"):
+            raise ValueError(f"filter {self.filter!r}: 'post' (the reference's post-pass over the 2k best rows) or "
+                             "'exact' (the exact top-k among the filter_ids rows)")
         if self.metric not in ("cosine", "ip", "inner_product"):
             raise ValueError(f"metric {self.metric!r}: only the cosine / inner-product path is B200-native "
                              "(IndexFlatL2 is outside the hot path)")
@@ -348,16 +448,24 @@ class B200FlatIndex(IndexBase):
 
     def search(self, query_embeddings: np.ndarray, k: int = 10,
                filter_ids: Optional[List[str]] = None) -> Tuple[List[List[str]], List[List[float]]]:
-        """FaissIndex.search (retrieval.py:141-197): exact top-k, rows mapped to item ids; `filter_ids` is the
-        reference's POST-filter over the k_search = min(2k, N) best rows (it may return fewer than k ids)."""
+        """FaissIndex.search (retrieval.py:141-197): exact top-k, rows mapped to item ids.  `filter_ids` under config
+        "filter": "post" (default) is the reference's POST-filter over the k_search = min(2k, N) best rows (it may return
+        fewer than k ids); under "exact" the result is the exact top-k among the rows of the known filter_ids
+        (min(k, |allowed rows|) ids per query; unknown ids are ignored)."""
         if self.index is None:
             raise ValueError("Index not built yet")
         if not (torch.is_tensor(query_embeddings) and query_embeddings.is_cuda):   # device tensors skip the host round trip
             query_embeddings = np.asarray(query_embeddings).astype(np.float32)
         if len(query_embeddings.shape) == 1:
             query_embeddings = query_embeddings.reshape(1, -1)
-        k_search = min(k * 2, self.current_size) if filter_ids else k
-        distances, indices = self.index.search(query_embeddings, k_search, normalize=(self.metric == "cosine"))
+        exact = filter_ids is not None and self.filter == "exact"
+        if exact:
+            rows = np.fromiter((self.reverse_id_map[x] for x in set(filter_ids) if x in self.reverse_id_map), np.int64)
+            distances, indices = self.index.search(query_embeddings, k, normalize=(self.metric == "cosine"),
+                                                   sel=self.index.row_filter(rows=rows))
+        else:
+            k_search = min(k * 2, self.current_size) if filter_ids else k
+            distances, indices = self.index.search(query_embeddings, k_search, normalize=(self.metric == "cosine"))
         if self.current_size == 0:
             return [[] for _ in range(len(indices))], [[] for _ in range(len(indices))]
         names = self._names()
@@ -365,7 +473,7 @@ class B200FlatIndex(IndexBase):
         safe = np.where(keep, indices, 0)
         keep &= self._mapped[safe]
         picked = names[safe]
-        if filter_ids is not None:                                             # [] filters everything out, as the reference
+        if filter_ids is not None and not exact:                               # [] filters everything out, as the reference
             member = set(filter_ids).__contains__                              # one C-level pass over the candidates
             keep &= np.frompyfunc(member, 1, 1)(picked).astype(bool)
         if keep.all():
