@@ -104,6 +104,28 @@ int b200rec_flat_ip_topk_fanout(const void* catalogue, int64_t N, int64_t ld, co
 int b200rec_topk_sample_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
                                int k_out, int shards, int n_dst, void* const* dst_vals, void* workspace,
                                size_t workspace_bytes, void* stream);
+/* Filtered row-shard steps (row-sharded filtered search; every shard passes through both exchanges, so neither step
+ * fails for lack of work: it stores padding rows to every destination instead).
+ * b200rec_topk_sample_filtered[_fanout]: b200rec_topk_sample over the rows allowed by allow_bits (bitmap as in
+ * b200rec_flat_ip_topk_filtered; disallowed sampled rows count as -inf), or over the whole catalogue when allow_bits is
+ * NULL (a compacted catalogue).  When no row is allowed (N == 0 or allow_n == 0) or the shape has no sampling pass, every
+ * destination gets -FLT_MAX rows, which bound nothing from below.
+ * b200rec_flat_ip_topk_filtered_fanout: the local top-k of a row shard starting from tau_init (nullable), stored to the
+ * n_dst destinations.  Exactly one of allow_bits (bitmap path; ids = row + row_offset) and remap_rows (compacted
+ * catalogue path: N = n_remap compacted rows, row j is local row remap_rows[j], ids = remap_rows[j] + row_offset, mapped
+ * inside the select kernel) is given.  No allowed row (N == 0 or allow_n == 0): -FLT_MAX / -1 rows everywhere. */
+int b200rec_topk_sample_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
+                                 int k_out, int shards, const uint32_t* allow_bits, int64_t allow_n, float* out_vals,
+                                 void* workspace, size_t workspace_bytes, void* stream);
+int b200rec_topk_sample_filtered_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                        int k, int k_out, int shards, const uint32_t* allow_bits, int64_t allow_n,
+                                        int n_dst, void* const* dst_vals, void* workspace, size_t workspace_bytes,
+                                        void* stream);
+int b200rec_flat_ip_topk_filtered_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                         int k, int64_t row_offset, const uint32_t* allow_bits, int64_t allow_n,
+                                         const int64_t* remap_rows, int64_t n_remap, const float* tau_init, int n_dst,
+                                         void* const* dst_scores, void* const* dst_ids, void* workspace,
+                                         size_t workspace_bytes, void* stream);
 /* k-way merge of `parts` candidate lists [parts][Q][k_in] (id < 0 = empty, ids < 2^32) into the global top k_out under
  * the same order: the exchange step after the all-gather of per-GPU results.  *_part_stride = element distance
  * between consecutive parts (0 = dense, Q*k_in); non-dense strides let one all-gather carry scores and ids together. */

@@ -825,8 +825,10 @@ struct OutFan {
   int64_t* i[FAN_MAX];
 };
 
-__device__ __forceinline__ void write_result(const uint64_t* skeys, int k_out, int64_t row_offset, float* out_s,
-                                             int64_t* out_i) {
+// remap (nullable): the select ran over a compacted catalogue whose row j is local row remap[j] (compact filtered search
+// of a row shard); the id leaves the kernel already mapped, because on the peer path it is stored straight to the peers
+__device__ __forceinline__ void write_result(const uint64_t* skeys, int k_out, int64_t row_offset, const int64_t* remap,
+                                             float* out_s, int64_t* out_i) {
   for (int i = threadIdx.x; i < k_out; i += FIN_THREADS) {
     const uint64_t key = skeys[i];
     if (key == 0ull) {
@@ -834,7 +836,8 @@ __device__ __forceinline__ void write_result(const uint64_t* skeys, int k_out, i
       out_i[i] = -1;
     } else {
       out_s[i] = ord_f32((uint32_t)(key >> 32));
-      out_i[i] = (int64_t)(~(uint32_t)key) + row_offset;
+      const uint32_t row = ~(uint32_t)key;
+      out_i[i] = (remap != nullptr ? __ldg(remap + row) : (int64_t)row) + row_offset;
     }
   }
 }
@@ -863,7 +866,7 @@ __global__ void __launch_bounds__(FIN_THREADS)
 topk_final_kernel(const StreamGeom g, int v2, int qs /*queries per supertile*/, int slots /*per CTA*/,
                   const uint64_t* __restrict__ tlists, const QMeta* __restrict__ meta,
                   const uint64_t* __restrict__ lists, const uint32_t* __restrict__ left, int cap, int k, int P,
-                  int stage_cap, int64_t row_offset, const OutFan fan) {
+                  int stage_cap, int64_t row_offset, const int64_t* __restrict__ remap, const OutFan fan) {
   extern __shared__ uint64_t fin_smem[];
   __shared__ uint32_t hist[256];
   __shared__ int s_misc[8];
@@ -913,7 +916,7 @@ topk_final_kernel(const StreamGeom g, int v2, int qs /*queries per supertile*/, 
   __syncthreads();
   block_select_sort(ld, n, k, fin_smem, P, hist, s_misc, fin_smem + P, stage_cap);
   for (int d = 0; d < fan.n; ++d)
-    write_result(fin_smem, k, row_offset, fan.s[d] + (size_t)q * k, fan.i[d] + (size_t)q * k);
+    write_result(fin_smem, k, row_offset, remap, fan.s[d] + (size_t)q * k, fan.i[d] + (size_t)q * k);
 }
 
 // per-query k largest group maxima of the sampling pass (descending; -FLT_MAX padding): what shards exchange so that
@@ -937,6 +940,16 @@ sample_topk_kernel(const float* __restrict__ S, int m, int k, int P, int stage_c
     const float v = key == 0ull ? -FLT_MAX : ord_f32((uint32_t)(key >> 32));
     for (int d = 0; d < fan.n; ++d) fan.s[d][(size_t)q * k + i] = v;
   }
+}
+
+// n values `s` (and ids `id` where the destination has an id array) stored to every fan-out destination: the padding rows
+// a row shard with nothing to sample or search still owes every peer's gather buffer
+__global__ void __launch_bounds__(256) fan_fill_kernel(const OutFan fan, int64_t n, float s, int64_t id) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+    for (int d = 0; d < fan.n; ++d) {
+      fan.s[d][i] = s;
+      if (fan.i[d] != nullptr) fan.i[d][i] = id;
+    }
 }
 
 // k-th largest of the `parts` x k_in pooled sample maxima of every query (parts-major layout [parts][Q][k_in], as the
@@ -1019,7 +1032,7 @@ topk_merge_kernel(const float* __restrict__ scores, const int64_t* __restrict__ 
   ld.i_stride = (size_t)i_stride;
   ld.k_in = k_in;
   block_select_sort(ld, parts * k_in, k_out, fin_smem, P, hist, s_misc, fin_smem + P, stage_cap);
-  write_result(fin_smem, k_out, 0, out_scores + (size_t)q * k_out, out_ids + (size_t)q * k_out);
+  write_result(fin_smem, k_out, 0, nullptr, out_scores + (size_t)q * k_out, out_ids + (size_t)q * k_out);
 }
 
 // Initial thresholds from a strided catalogue sample: tau0[q] = (a lower bound of) the k-th largest of the m sampled
@@ -1265,7 +1278,8 @@ template <int NQ, int BN, int V2, bool DBG>
 static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
                        int k, int64_t row_offset, const int64_t* excl_indptr, const int32_t* excl_rows,
                        const uint32_t* allow, int64_t allow_n, float* out_scores, int64_t* out_ids, void* workspace,
-                       cudaStream_t st, const float* tau_init, float* sample_vals_out, const OutFan* fan_in) {
+                       cudaStream_t st, const float* tau_init, float* sample_vals_out, const OutFan* fan_in,
+                       const int64_t* remap) {
   OutFan fan;
   if (fan_in != nullptr) {
     fan = *fan_in;
@@ -1370,7 +1384,7 @@ static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int6
   const int fin_stage = P <= 1024 ? 1024 : 0;  // T + leftovers of a query usually are a few hundred keys
   topk_final_kernel<<<(unsigned)Q, FIN_THREADS, (P + fin_stage) * sizeof(uint64_t), st>>>(
       p.g, V2, V2 == 2 ? 512 : (V2 == 1 ? 256 : 128 * NQ), V2 ? S2_SLOTS : 128 * NQ, ea.tlists, ea.meta, ea.lists, ea.left, p.cap,
-      k, P, fin_stage, row_offset, fan);
+      k, P, fin_stage, row_offset, remap, fan);
   B200_LAUNCH_OK("topk_final_kernel");
   return 0;
 }
@@ -1441,7 +1455,7 @@ static int topk_dispatch(const void* catalogue, int64_t N, int64_t ld, const voi
                          int64_t row_offset, const int64_t* exclude_indptr, const int32_t* exclude_rows,
                          const uint32_t* allow, int64_t allow_n, const float* tau_init, float* out_scores,
                          int64_t* out_ids, float* sample_vals_out,
-                         int sample_k_out, int shards, const b200::OutFan* fan,
+                         int sample_k_out, int shards, const b200::OutFan* fan, const int64_t* remap,
                          void* workspace, size_t workspace_bytes, void* stream) {
   using namespace b200;
   TopkPlan p;
@@ -1452,7 +1466,7 @@ static int topk_dispatch(const void* catalogue, int64_t N, int64_t ld, const voi
   if ((exclude_indptr == nullptr) != (exclude_rows == nullptr)) return fail("topk: exclusion CSR needs both arrays");
   if (sample_vals_out != nullptr && p.sample_m == 0) return fail("topk_sample: catalogue too small for a sampling pass");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-#define B200_TOPK_ARGS p, catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, allow, allow_n, out_scores, out_ids, workspace, st, tau_init, sample_vals_out, fan
+#define B200_TOPK_ARGS p, catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, allow, allow_n, out_scores, out_ids, workspace, st, tau_init, sample_vals_out, fan, remap
   if (knobs().debug != 0 || knobs().stream_stats || knobs().stats_unit >= 0) {  // development instantiation
     if (p.v2 == 2) return launch_topk<2, 128, 2, true>(B200_TOPK_ARGS);
     if (p.v2 == 1) return launch_topk<2, 128, 1, true>(B200_TOPK_ARGS);
@@ -1474,7 +1488,7 @@ extern "C" int b200rec_flat_ip_topk(const void* catalogue, int64_t N, int64_t ld
                                     size_t workspace_bytes, void* stream) {
   if (!catalogue || !queries || !out_scores || !out_ids || !workspace) return b200::fail("topk: null pointer");
   return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, nullptr, 0, tau_init,
-                       out_scores, out_ids, nullptr, k, 1, nullptr, workspace, workspace_bytes, stream);
+                       out_scores, out_ids, nullptr, k, 1, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
@@ -1485,7 +1499,7 @@ extern "C" int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, i
     return b200::fail("topk_filtered: null pointer");
   if (allow_n < 0) return b200::fail("topk_filtered: allow_n must be >= 0");
   return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, allow_bits, allow_n < N ? allow_n : N,
-                       nullptr, out_scores, out_ids, nullptr, k, 1, nullptr, workspace, workspace_bytes, stream);
+                       nullptr, out_scores, out_ids, nullptr, k, 1, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int b200rec_topk_sample(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
@@ -1494,7 +1508,7 @@ extern "C" int b200rec_topk_sample(const void* catalogue, int64_t N, int64_t ld,
   if (!catalogue || !queries || !out_vals || !workspace) return b200::fail("topk_sample: null pointer");
   if (k_out < 1 || k_out > k) return b200::fail("topk_sample: k_out must be in [1, k]");
   return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, out_vals, k_out,
-                       shards < 1 ? 1 : shards, nullptr, workspace, workspace_bytes, stream);
+                       shards < 1 ? 1 : shards, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
 static int make_fan(b200::OutFan& fan, int n_dst, void* const* dst_scores, void* const* dst_ids, bool want_ids) {
@@ -1517,7 +1531,7 @@ extern "C" int b200rec_flat_ip_topk_fanout(const void* catalogue, int64_t N, int
   b200::OutFan fan;
   if (make_fan(fan, n_dst, dst_scores, dst_ids, true)) return 1;
   return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, nullptr, 0, tau_init, fan.s[0], fan.i[0], nullptr, k,
-                       1, &fan, workspace, workspace_bytes, stream);
+                       1, &fan, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int b200rec_topk_sample_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
@@ -1528,7 +1542,7 @@ extern "C" int b200rec_topk_sample_fanout(const void* catalogue, int64_t N, int6
   b200::OutFan fan;
   if (make_fan(fan, n_dst, dst_vals, nullptr, false)) return 1;
   return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, nullptr, 0, nullptr, nullptr, nullptr, fan.s[0], k_out,
-                       shards < 1 ? 1 : shards, &fan, workspace, workspace_bytes, stream);
+                       shards < 1 ? 1 : shards, &fan, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int b200rec_topk_has_sample(int64_t N, int64_t ld, int64_t Q, int k) {
@@ -1569,4 +1583,86 @@ extern "C" int b200rec_topk_merge(const float* scores, const int64_t* ids, int p
       (long long)(ids_part_stride > 0 ? ids_part_stride : Q * k_in), out_scores, out_ids);
   B200_LAUNCH_OK("topk_merge_kernel");
   return 0;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// filtered row-shard steps: every shard takes part in every exchange, so a shard that has nothing to sample or search
+// (no allowed rows, or a shape without a sampling pass) stores padding rows instead of failing
+// ---------------------------------------------------------------------------------------------------------------
+static int fan_fill(const b200::OutFan& fan, int64_t n, float s, int64_t id, void* stream) {
+  using namespace b200;
+  const int64_t blocks = (n + 255) / 256;
+  const int grid = (int)(blocks < 4 * (int64_t)num_sms() ? (blocks > 0 ? blocks : 1) : 4 * (int64_t)num_sms());
+  fan_fill_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(fan, n, s, id);
+  B200_LAUNCH_OK("fan_fill_kernel");
+  return 0;
+}
+
+static int sample_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k, int k_out,
+                           int shards, const uint32_t* allow_bits, int64_t allow_n, const b200::OutFan& fan,
+                           void* workspace, size_t workspace_bytes, void* stream) {
+  using namespace b200;
+  if (Q < 1) return fail("topk_sample_filtered: Q must be >= 1");
+  if (k < 1 || k > 2048) return fail("topk_sample_filtered: k must be in [1, 2048] (got %d)", k);
+  if (k_out < 1 || k_out > k) return fail("topk_sample_filtered: k_out must be in [1, k]");
+  if (N < 0 || allow_n < 0) return fail("topk_sample_filtered: N and allow_n must be >= 0");
+  shards = shards < 1 ? 1 : shards;
+  const int64_t an = allow_bits != nullptr ? (allow_n < N ? allow_n : N) : N;
+  bool pad = N == 0 || an == 0;
+  if (!pad) {
+    TopkPlan p;
+    if (plan_topk(p, N, ld, Q, k, shards)) return 1;
+    if (p.sample_m == 0 && plan_topk(p, N, ld, Q, k)) return 1;
+    pad = p.sample_m == 0;
+  }
+  if (pad) return fan_fill(fan, Q * k_out, -FLT_MAX, 0, stream);
+  if (!catalogue || !workspace) return fail("topk_sample_filtered: null catalogue or workspace");
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, 0, nullptr, nullptr, allow_bits, an, nullptr, nullptr, nullptr,
+                       fan.s[0], k_out, shards, &fan, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b200rec_topk_sample_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                            int k, int k_out, int shards, const uint32_t* allow_bits, int64_t allow_n,
+                                            float* out_vals, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!queries || !out_vals) return b200::fail("topk_sample_filtered: null pointer");
+  b200::OutFan fan;
+  fan.n = 1;
+  fan.s[0] = out_vals;
+  fan.i[0] = nullptr;
+  return sample_filtered(catalogue, N, ld, queries, Q, k, k_out, shards, allow_bits, allow_n, fan, workspace,
+                         workspace_bytes, stream);
+}
+
+extern "C" int b200rec_topk_sample_filtered_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries,
+                                                   int64_t Q, int k, int k_out, int shards, const uint32_t* allow_bits,
+                                                   int64_t allow_n, int n_dst, void* const* dst_vals, void* workspace,
+                                                   size_t workspace_bytes, void* stream) {
+  if (!queries) return b200::fail("topk_sample_filtered: null pointer");
+  b200::OutFan fan;
+  if (make_fan(fan, n_dst, dst_vals, nullptr, false)) return 1;
+  return sample_filtered(catalogue, N, ld, queries, Q, k, k_out, shards, allow_bits, allow_n, fan, workspace,
+                         workspace_bytes, stream);
+}
+
+extern "C" int b200rec_flat_ip_topk_filtered_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries,
+                                                    int64_t Q, int k, int64_t row_offset, const uint32_t* allow_bits,
+                                                    int64_t allow_n, const int64_t* remap_rows, int64_t n_remap,
+                                                    const float* tau_init, int n_dst, void* const* dst_scores,
+                                                    void* const* dst_ids, void* workspace, size_t workspace_bytes,
+                                                    void* stream) {
+  using namespace b200;
+  if (!queries) return fail("topk_filtered_fanout: null pointer");
+  if ((allow_bits == nullptr) == (remap_rows == nullptr))
+    return fail("topk_filtered_fanout: exactly one of allow_bits and remap_rows must be given");
+  OutFan fan;
+  if (make_fan(fan, n_dst, dst_scores, dst_ids, true)) return 1;
+  if (Q < 1) return fail("topk_filtered_fanout: Q must be >= 1");
+  if (k < 1 || k > 2048) return fail("topk_filtered_fanout: k must be in [1, 2048] (got %d)", k);
+  if (N < 0 || allow_n < 0) return fail("topk_filtered_fanout: N and allow_n must be >= 0");
+  if (remap_rows != nullptr && n_remap != N) return fail("topk_filtered_fanout: n_remap must equal N (one row per compacted row)");
+  const int64_t an = allow_bits != nullptr ? (allow_n < N ? allow_n : N) : N;
+  if (N == 0 || an == 0) return fan_fill(fan, Q * k, -FLT_MAX, -1, stream);
+  if (!catalogue || !workspace) return fail("topk_filtered_fanout: null catalogue or workspace");
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, allow_bits, an, tau_init, fan.s[0],
+                       fan.i[0], nullptr, k, 1, &fan, remap_rows, workspace, workspace_bytes, stream);
 }

@@ -14,6 +14,7 @@ import os
 import inspect
 from typing import Callable, Optional, Tuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -23,6 +24,35 @@ def shard_bounds(n_total: int, world: int, rank: int) -> Tuple[int, int]:
     base, rem = divmod(n_total, world)
     lo = rank * base + min(rank, rem)
     return lo, lo + base + (1 if rank < rem else 0)
+
+
+def shard_filter_rows(lo: int, n: int, rows=None, mask=None) -> np.ndarray:
+    """Local rows (ascending, in [0, n)) of the shard that holds global rows [lo, lo + n), from a filter over GLOBAL rows:
+    `rows` (int array; rows outside the shard and duplicates are dropped) or `mask` (1-D bool array over the global rows;
+    a mask shorter than the catalogue leaves the missing tail not allowed, entries past the catalogue are owned by no
+    shard)."""
+    if (rows is None) == (mask is None):
+        raise ValueError("row_filter takes exactly one of rows= or mask=")
+    if mask is not None:
+        m = np.asarray(mask.cpu() if torch.is_tensor(mask) else mask)
+        if m.dtype != np.bool_ or m.ndim != 1:
+            raise ValueError("mask must be a 1-D bool array over the global rows")
+        return np.flatnonzero(m[lo: lo + n])
+    r = np.asarray(rows.cpu() if torch.is_tensor(rows) else rows).reshape(-1)
+    if r.size and not np.issubdtype(r.dtype, np.integer):
+        raise ValueError("rows must be an integer array")
+    r = r.astype(np.int64, copy=False) - lo
+    return np.unique(r[(r >= 0) & (r < n)])
+
+
+class ShardedRowFilter:
+    """This rank's part of a row filter over the GLOBAL rows of a ShardedFlatIndex (`ShardedFlatIndex.row_filter`):
+    `local` is the filter of the local shard (a retrieval.RowFilter over its local rows), which the shard's filtered
+    sample and search steps receive.  Every rank must build it from the same global row set, as every rank passes the
+    same queries; building it needs no collective."""
+
+    def __init__(self, local):
+        self.local = local
 
 
 def _world() -> Tuple[int, int]:
@@ -99,6 +129,9 @@ class ShardedFlatIndex:
     local_sample(q, k[, k_out, shards]) -> [Q,k_out] scores of DISTINCT local rows per query, or None (optional).  When given, shards
         all-gather these and every shard starts from the k-th best of the union: a lower bound of the GLOBAL k-th
         score, so each GPU only collects candidates that can still reach the global top-k.
+    Filtered search (`search(..., sel=ShardedRowFilter)`) calls local_search(q, k, tau, out, sel=local filter) and
+    local_sample(q, k, k_out, shards, sel=local filter); the filtered sampler always returns [Q,k_out] (padding rows of
+    -FLT_MAX, or anything <= every real score, where it has nothing to sample).
     """
 
     def __init__(self, local_search: Callable, merge: Callable, group=None, local_sample: Optional[Callable] = None):
@@ -119,13 +152,17 @@ class ShardedFlatIndex:
     def from_device_index(cls, index, group=None, peer_exchange: bool = True) -> "ShardedFlatIndex":
         from . import kernels as K
 
-        def local(q_op, k, tau=None, out=None):
+        def local(q_op, k, tau=None, out=None, sel=None):
+            if sel is not None:
+                return index.search_filtered_shard(q_op, k, sel, tau, out=out)
             return index.search_device(q_op, k, tau_init=tau, out=out)
 
         def merge(s, i, k):
             return K.topk_merge(s, i, k)
 
-        def sample(q_op, k, k_out=None, shards=1):
+        def sample(q_op, k, k_out=None, shards=1, sel=None):
+            if sel is not None:
+                return index.sample_filtered(q_op, k, k if k_out is None else k_out, shards, sel)
             if not index.has_sample_pass(q_op.shape[0], k):
                 return None
             return index.sample_device(q_op, k, k_out, shards)
@@ -135,6 +172,18 @@ class ShardedFlatIndex:
         obj.peer_index = index
         obj.use_peer_exchange = bool(peer_exchange)
         return obj
+
+    def row_filter(self, rows=None, mask=None) -> ShardedRowFilter:
+        """Row filter over the GLOBAL rows held now (`FlatIPDeviceIndex.row_filter` semantics: `rows` int array with
+        out-of-range and duplicate rows ignored, or `mask` bool array with a missing tail not allowed; rows added later
+        are not allowed).  Every rank must pass the same global set; each keeps the slice of its own shard.  Pass it as
+        `sel=` to search / search_stream / search_numpy.  bf16 storage only."""
+        ix = self.peer_index
+        if ix is None:
+            raise RuntimeError("row_filter needs a ShardedFlatIndex built by from_device_index")
+        if ix.storage != "bf16":
+            raise ValueError("row-sharded filtered search needs bf16 storage (the index of this shard stores fp32)")
+        return ShardedRowFilter(ix.row_filter(rows=shard_filter_rows(ix.row_offset, ix.ntotal, rows, mask)))
 
     def _peer(self, q: int, k: int, world: int, device):
         """Peer gather buffers for this shape, or None when symmetric memory is unavailable / a shard has no sampling
@@ -157,13 +206,19 @@ class ShardedFlatIndex:
             self._ids_cache[key] = px if int(flag.item()) == 1 else None
         return self._ids_cache[key]
 
-    def _search_peer(self, px: "_PeerExchange", queries, k: int, world: int):
+    def _search_peer(self, px: "_PeerExchange", queries, k: int, world: int, sel=None):
         ix = self.peer_index
-        ix.sample_fanout(queries, k, px.tau_all.shape[2], world, px.tau_dst)     # (1) sample -> every gather buffer
+        if sel is None:
+            ix.sample_fanout(queries, k, px.tau_all.shape[2], world, px.tau_dst)  # (1) sample -> every gather buffer
+        else:                                           # allowed rows only; padding rows where there is nothing to sample
+            ix.sample_filtered(queries, k, px.tau_all.shape[2], world, sel, dst=px.tau_dst)
         px.barrier(0)
         from . import kernels as K
         tau = K.topk_pooled_kth(px.tau_all, k)                                   # (2) k-th best of the pooled sample
-        ix.search_fanout(queries, k, tau, px.s_dst, px.i_dst)                    # (3) local top-k -> every gather buffer
+        if sel is None:
+            ix.search_fanout(queries, k, tau, px.s_dst, px.i_dst)                # (3) local top-k -> every gather buffer
+        else:
+            ix.search_filtered_shard(queries, k, sel, tau, dst=(px.s_dst, px.i_dst))
         px.barrier(1)
         return self.merge(px.s_all, px.i_all, k)                                 # (4) k-way select
 
@@ -172,26 +227,39 @@ class ShardedFlatIndex:
         """Sample maxima each shard contributes to the threshold exchange.  The union must hold >= k distinct rows for
         its k-th best to bound the global k-th score from below; a shard owns about k/world of the union's top k
         (binomial), so k/world + 4 sigma + 8 keeps the bound as tight as exchanging k per shard at a fraction of the
-        bytes (world 8, k 100: 32 instead of 100)."""
+        bytes (world 8, k 100: 32 instead of 100).
+
+        Filtered search pools the same widths, sampled over the allowed rows only, and a shard with nothing to sample
+        (no allowed row, or no sampling pass for its shape) contributes padding rows of -FLT_MAX or -inf.  The bound
+        still holds: if the pool holds at least k values that are scores of distinct allowed rows, its k-th best is <=
+        the k-th best allowed score of the whole catalogue; if it holds fewer, its k-th best is a padding value, below
+        every real score.  Padding and skew (all allowed rows on one shard, which then exchanges only k' of them) only
+        loosen the bound, down to no pruning at all, so no shard has to agree with the others on whether to sample."""
         if world <= 1:
             return k
         mean = -(-k // world)
         return min(k, mean + 4 * int(mean ** 0.5) + 8)
 
-    def _shared_thresholds(self, queries, k: int, world: int):
-        """k-th best of the union of every shard's sample: [Q] lower bounds of the global k-th score (or None)."""
+    def _shared_thresholds(self, queries, k: int, world: int, sel=None):
+        """k-th best of the union of every shard's sample: [Q] lower bounds of the global k-th score (or None).
+        With a row filter `sel` (this shard's local filter): of the global k-th ALLOWED score.  Every shard then always
+        contributes a [Q, k'] sample, padded where it has nothing to sample (see exchange_width), so the filtered call
+        needs no agreement round."""
         kx = self.exchange_width(k, world)
-        vals = self.local_sample(queries, k, kx, world) if self._sample_takes_width else self.local_sample(queries, k)
-        shape_key = ("use", int(queries.shape[0]), k)
-        if shape_key not in self._ids_cache:
-            # every shard must take the same branch: agree once per (batch, k) shape (one host sync, then cached)
-            flag = torch.tensor([0 if vals is None else 1], dtype=torch.int32)
-            if dist.get_backend(self.group) == "nccl":
-                flag = flag.cuda()
-            dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
-            self._ids_cache[shape_key] = int(flag.item()) == 1
-        if not self._ids_cache[shape_key] or vals is None:
-            return None
+        if sel is not None:
+            vals = self.local_sample(queries, k, kx, world, sel=sel)
+        else:
+            vals = self.local_sample(queries, k, kx, world) if self._sample_takes_width else self.local_sample(queries, k)
+            shape_key = ("use", int(queries.shape[0]), k)
+            if shape_key not in self._ids_cache:
+                # every shard must take the same branch: agree once per (batch, k) shape (one host sync, then cached)
+                flag = torch.tensor([0 if vals is None else 1], dtype=torch.int32)
+                if dist.get_backend(self.group) == "nccl":
+                    flag = flag.cuda()
+                dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
+                self._ids_cache[shape_key] = int(flag.item()) == 1
+            if not self._ids_cache[shape_key] or vals is None:
+                return None
         q, kv = vals.shape
         key = (world, q, kv, str(vals.device))
         if key not in self._ids_cache:  # any distinct ids will do: only the merged scores are used
@@ -202,15 +270,19 @@ class ShardedFlatIndex:
         top, _ = self.merge(allv.view(world, q, kv), ids, k)
         return top[:, k - 1].contiguous()
 
-    def search(self, queries, k: int):
+    def search(self, queries, k: int, sel: Optional[ShardedRowFilter] = None):
+        """Global top-k on every rank.  `sel` (from row_filter): the global exact top-k among the allowed rows, in the
+        order and padding of the single-index filtered search (score desc, global row asc, -1 / -FLT_MAX past them)."""
         world, _ = _world()
+        lsel = None if sel is None else sel.local
+        kw = {} if sel is None else {"sel": lsel}
         if world == 1:
-            return self.local_search(queries, k)
+            return self.local_search(queries, k, **kw)
         if self.peer_index is not None and self.use_peer_exchange:
             px = self._peer(int(queries.shape[0]), k, world, queries.device)
             if px is not None:
-                return self._search_peer(px, queries, k, world)
-        tau = self._shared_thresholds(queries, k, world) if self.local_sample is not None else None
+                return self._search_peer(px, queries, k, world, lsel)
+        tau = self._shared_thresholds(queries, k, world, lsel) if self.local_sample is not None else None
         q = int(queries.shape[0])
         if self.packed_exchange and (q * k) % 2 == 0:
             # one all-gather carries scores and ids: each rank's chunk is [q*k fp32 | q*k int64]
@@ -222,13 +294,16 @@ class ShardedFlatIndex:
             mine, everyone = self._ids_cache[key]
             s_view = mine[: 4 * q * k].view(torch.float32).view(q, k)
             i_view = mine[4 * q * k:].view(torch.int64).view(q, k)
-            self.local_search(queries, k, tau, (s_view, i_view))
+            self.local_search(queries, k, tau, (s_view, i_view), **kw)
             dist.all_gather_into_tensor(everyone, mine, group=self.group)
             chunks = everyone.view(world, 12 * q * k)
             gs = chunks[:, : 4 * q * k].view(torch.float32).view(world, q, k)
             gi = chunks[:, 4 * q * k:].view(torch.int64).view(world, q, k)
             return self.merge(gs, gi, k)
-        s, i = self.local_search(queries, k, tau) if tau is not None else self.local_search(queries, k)
+        if sel is not None:
+            s, i = self.local_search(queries, k, tau, **kw)
+        else:
+            s, i = self.local_search(queries, k, tau) if tau is not None else self.local_search(queries, k)
         gs = torch.empty((world * q, s.shape[1]), dtype=s.dtype, device=s.device)
         gi = torch.empty((world * q, i.shape[1]), dtype=i.dtype, device=i.device)
         dist.all_gather_into_tensor(gs, s.contiguous(), group=self.group)
@@ -237,10 +312,10 @@ class ShardedFlatIndex:
 
 
     # ------------------------------------------------------------------ host-facing calls (faiss array contract)
-    def _host_pipe(self, k: int, normalize: bool, share: bool):
+    def _host_pipe(self, k: int, normalize: bool, share: bool, filtered: bool = False):
         from .retrieval import HostPipeline
         world, rank = _world()
-        key = ("pipe", k, normalize, share)
+        key = ("pipe", k, normalize, share, filtered)    # a filtered stream never runs the unfiltered pipe's search
         if key not in self._ids_cache:
             rows = None
             if share and world > 1:     # every replica returns the answers of ITS contiguous share of the query batch
@@ -248,19 +323,32 @@ class ShardedFlatIndex:
             self._ids_cache[key] = HostPipeline(self.peer_index, k, normalize, lambda q_op, kk: self.search(q_op, kk), rows)
         return self._ids_cache[key]
 
-    def search_stream(self, batches, k: int, normalize: bool = False, share_results: bool = False):
+    def search_stream(self, batches, k: int, normalize: bool = False, share_results: bool = False,
+                      sel: Optional[ShardedRowFilter] = None):
         """`FlatIPDeviceIndex.search_stream` over the row-sharded catalogue: every replica passes the same HOST query
         batches (numpy) and gets faiss-shaped (D, I) numpy pairs with GLOBAL row ids.  share_results=True copies back
         only this replica's contiguous share of the queries (rows shard_bounds(nq, world, rank)), which is what a
-        replicated serving tier needs; False returns the full result on every replica."""
+        replicated serving tier needs; False returns the full result on every replica.  `sel` (row_filter): the exact
+        top-k among the allowed rows."""
         if self.peer_index is None:
             raise RuntimeError("search_stream needs a ShardedFlatIndex built by from_device_index")
-        pipe = self._host_pipe(k, normalize, share_results)
+        pipe = self._host_pipe(k, normalize, share_results, sel is not None)
+        if sel is not None:
+            batches = self._with_filter(pipe, batches, sel)
         return self.peer_index.search_stream(batches, k, normalize, device_search=pipe)
 
-    def search_numpy(self, q, k: int, normalize: bool = False, share_results: bool = False):
+    def _with_filter(self, pipe, batches, sel: ShardedRowFilter):
+        """The batches of one filtered stream, pointing the (shared) filtered pipe's device search at `sel` right before
+        each batch is submitted: every batch is searched with the filter of the stream it belongs to."""
+        search = lambda q_op, kk: self.search(q_op, kk, sel=sel)   # noqa: E731
+        for q in batches:
+            pipe.device_search = search
+            yield q
+
+    def search_numpy(self, q, k: int, normalize: bool = False, share_results: bool = False,
+                     sel: Optional[ShardedRowFilter] = None):
         """One blocking faiss-shaped call: numpy queries in, (D, I) numpy out."""
-        for out in self.search_stream([q], k, normalize, share_results):
+        for out in self.search_stream([q], k, normalize, share_results, sel):
             return out
 
 

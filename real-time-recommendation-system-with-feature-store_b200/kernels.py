@@ -176,6 +176,47 @@ def topk_sample_fanout(catalogue: torch.Tensor, queries: torch.Tensor, k: int, k
                                                workspace.numel(), N.stream()), "topk_sample_fanout")
 
 
+def topk_sample_filtered(catalogue: Optional[torch.Tensor], queries: torch.Tensor, k: int, k_out: int, shards: int,
+                         allow_bits: Optional[torch.Tensor], allow_n: int, workspace: Optional[torch.Tensor],
+                         dst_vals=None) -> Optional[torch.Tensor]:
+    """Sampling pass of one row shard of a filtered search: the k_out largest group maxima per query over the rows the
+    bitmap allows (allow_bits None: every row of `catalogue`, a compacted one).  -FLT_MAX rows when nothing is allowed or
+    the shape has no sampling pass.  dst_vals (device addresses): stored to every one of them, else returned [Q, k_out].
+    catalogue / workspace may be None when the shard holds no row."""
+    n = 0 if catalogue is None else catalogue.shape[0]
+    ld = queries.stride(0)
+    q = queries.shape[0]
+    ws_n = 0 if workspace is None else workspace.numel()
+    if dst_vals is None:
+        vals = torch.empty((q, k_out), dtype=torch.float32, device=queries.device)
+        N.check(N.lib().b200rec_topk_sample_filtered(N.ptr(catalogue), n, ld, N.ptr(queries), q, k, k_out, shards,
+                                                     N.ptr(allow_bits), allow_n, N.ptr(vals), N.ptr(workspace), ws_n,
+                                                     N.stream()), "topk_sample_filtered")
+        return vals
+    N.check(N.lib().b200rec_topk_sample_filtered_fanout(N.ptr(catalogue), n, ld, N.ptr(queries), q, k, k_out, shards,
+                                                        N.ptr(allow_bits), allow_n, len(dst_vals), _ptr_table(dst_vals),
+                                                        N.ptr(workspace), ws_n, N.stream()), "topk_sample_filtered_fanout")
+    return None
+
+
+def flat_ip_topk_filtered_fanout(catalogue: Optional[torch.Tensor], queries: torch.Tensor, k: int, row_offset: int,
+                                 allow_bits: Optional[torch.Tensor], allow_n: int, remap_rows: Optional[torch.Tensor],
+                                 tau_init: Optional[torch.Tensor], dst_scores, dst_ids,
+                                 workspace: Optional[torch.Tensor]) -> None:
+    """Local top-k of one row shard of a filtered search, from tau_init, stored to every (dst_scores[d], dst_ids[d]).
+    Exactly one of allow_bits (bitmap over `catalogue`) and remap_rows (int64: `catalogue` is compacted, its row j is local
+    row remap_rows[j]; the select kernel stores remap_rows[j] + row_offset) is given.  -1 / -FLT_MAX rows when nothing is
+    allowed; catalogue / workspace may then be None."""
+    n = 0 if catalogue is None else catalogue.shape[0]
+    n_remap = 0 if remap_rows is None else remap_rows.numel()
+    N.check(N.lib().b200rec_flat_ip_topk_filtered_fanout(N.ptr(catalogue), n, queries.stride(0), N.ptr(queries),
+                                                         queries.shape[0], k, row_offset, N.ptr(allow_bits), allow_n,
+                                                         N.ptr(remap_rows), n_remap, N.ptr(tau_init), len(dst_scores),
+                                                         _ptr_table(dst_scores), _ptr_table(dst_ids), N.ptr(workspace),
+                                                         0 if workspace is None else workspace.numel(), N.stream()),
+            "flat_ip_topk_filtered_fanout")
+
+
 def topk_has_sample(n: int, ld: int, q: int, k: int) -> bool:
     return bool(N.lib().b200rec_topk_has_sample(n, ld, q, k))
 

@@ -232,6 +232,52 @@ class FlatIPDeviceIndex:
             r = np.unique(r[(r >= 0) & (r < self.ntotal)])
         return RowFilter(self, r)
 
+    # ------------------------------------------------------------------ filtered row-shard steps (dist.ShardedFlatIndex)
+    def _shard_operand(self, sel: RowFilter, compact: Optional[bool]):
+        """(catalogue, allow_bits, allow_n, remap_rows) a filtered row-shard step runs over: the bitmap over the local
+        catalogue, or the compacted allowed rows with their local row list (compact = None: chosen from the LOCAL
+        allowed fraction, as search_device does).  No allowed row: (None, bits, 0, None), which the kernels answer with
+        padding rows."""
+        if self.storage != "bf16":
+            raise ValueError("row-sharded filtered search needs bf16 storage (an fp32-storage shard re-scores its "
+                             "candidates from fp32 rows, which the sharded exchange does not carry)")
+        if sel.index is not self:
+            raise ValueError("the row filter was built for another index")
+        if sel.n_allowed == 0:
+            return None, sel.bits, 0, None
+        if compact is None:
+            compact = sel.fraction < self.FILTER_COMPACT_BELOW
+        if compact:
+            return sel.compacted(), None, 0, sel.rows
+        return self._cat[: self.ntotal], sel.bits, sel.n_bits, None
+
+    def sample_filtered(self, q_op: torch.Tensor, k: int, k_out: int, shards: int, sel: RowFilter, dst=None,
+                        compact: Optional[bool] = None) -> Optional[torch.Tensor]:
+        """Sampling pass of a filtered row-sharded search: the k_out best group maxima per query over the allowed rows
+        only, sampled for `shards` pooled shards; -FLT_MAX rows when this shard has no allowed row or no sampling pass
+        for the shape.  Returned [nq, k_out], or stored to every address in `dst` (peer gather buffers)."""
+        cat, bits, allow_n, _ = self._shard_operand(sel, compact)
+        ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
+        return K.topk_sample_filtered(cat, q_op, k, k_out, shards, bits, allow_n, ws, dst)
+
+    def search_filtered_shard(self, q_op: torch.Tensor, k: int, sel: RowFilter, tau, out=None, dst=None,
+                              compact: Optional[bool] = None):
+        """Local exact top-k over the allowed rows from the pooled threshold `tau` ([nq] lower bounds of the GLOBAL k-th
+        allowed score, or None), global row ids (row_offset added, compact ids mapped back inside the select kernel),
+        -1 / -FLT_MAX padding.  Returns (D, I) (written into `out` when given), or stores the rows to every
+        (dst[0][d], dst[1][d]) address and returns None."""
+        cat, bits, allow_n, remap = self._shard_operand(sel, compact)
+        ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
+        if dst is not None:
+            K.flat_ip_topk_filtered_fanout(cat, q_op, k, self.row_offset, bits, allow_n, remap, tau, dst[0], dst[1], ws)
+            return None
+        nq = q_op.shape[0]
+        d, i = out if out is not None else (torch.empty((nq, k), dtype=torch.float32, device=self.device),
+                                            torch.empty((nq, k), dtype=torch.int64, device=self.device))
+        K.flat_ip_topk_filtered_fanout(cat, q_op, k, self.row_offset, bits, allow_n, remap, tau, [d.data_ptr()],
+                                       [i.data_ptr()], ws)
+        return d, i
+
     def search_device(self, q_op: torch.Tensor, k: int, exclude_indptr=None, exclude_rows=None, tau_init=None,
                       out=None, sel: Optional[RowFilter] = None):
         """q_op: bf16 operand [nq, ld] on the device -> (D, I) device tensors (written into `out` when given).
