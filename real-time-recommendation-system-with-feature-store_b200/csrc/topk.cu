@@ -1274,6 +1274,23 @@ static int plan_topk(TopkPlan& p, int64_t N, int64_t ld, int64_t Q, int k, int s
   return 0;
 }
 
+// the plan a search of one of `shards` pooled row shards runs with
+static int search_plan(TopkPlan& p, int64_t N, int64_t ld, int64_t Q, int k, int shards) {
+  if (plan_topk(p, N, ld, Q, k, shards)) return 1;
+  if (shards > 1 && p.sample_m == 0 && plan_topk(p, N, ld, Q, k)) return 1;  // pooled density too thin for this shard
+  return 0;
+}
+
+// hand a list over every ~k/4 candidates: each merge selects over k + list keys, so the threshold scales with k
+// (k = 1000: 7.6 ms per 1024-query batch at 32, 5.3 ms at 256).  Few queries and a large k (the serving loop's
+// top-1000 for <= 256 users): every unit feeds the same few queries, the merges serialise on those queries' locks and
+// a fresher threshold saves little, so lists are only handed over when full and the final select does the merging
+// (50 M x 64, k = 1000: Q = 1 4.44 -> 1.55 ms, Q = 128 5.07 -> 3.37 ms; at Q >= 512 the k/4 rule wins: 6.6 vs 8.2 ms).
+static int flush_for(const TopkPlan& p, int64_t Q, int k) {
+  const TopkKnobs& kn = knobs();
+  return kn.flush >= 0 ? kn.flush : ((k > 128 && Q <= 256) ? p.cap : (k / 4 > 32 ? (k / 4) / 32 * 32 : 32));
+}
+
 template <int NQ, int BN, int V2, bool DBG>
 static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
                        int k, int64_t row_offset, const int64_t* excl_indptr, const int32_t* excl_rows,
@@ -1306,12 +1323,7 @@ static int launch_topk(const TopkPlan& p, const void* catalogue, int64_t N, int6
   ea.allow_n = (uint32_t)allow_n;
   ea.k = k;
   ea.cap = p.cap;
-  // hand a list over every ~k/4 candidates: each merge selects over k + list keys, so the threshold scales with k
-  // (k = 1000: 7.6 ms per 1024-query batch at 32, 5.3 ms at 256).  Few queries and a large k (the serving loop's
-  // top-1000 for <= 256 users): every unit feeds the same few queries, the merges serialise on those queries' locks and
-  // a fresher threshold saves little, so lists are only handed over when full and the final select does the merging
-  // (50 M x 64, k = 1000: Q = 1 4.44 -> 1.55 ms, Q = 128 5.07 -> 3.37 ms; at Q >= 512 the k/4 rule wins: 6.6 vs 8.2 ms).
-  ea.flush = kn.flush >= 0 ? kn.flush : ((k > 128 && Q <= 256) ? p.cap : (k / 4 > 32 ? (k / 4) / 32 * 32 : 32));
+  ea.flush = flush_for(p, Q, k);
   ea.debug = kn.debug;
   ea.hsleep = kn.hsleep;
   void (*kern)(const CUtensorMap, const CUtensorMap, const StreamGeom, const TopkArgs);
@@ -1400,6 +1412,23 @@ extern "C" int b200rec_debug_reload_env(void) {
   return 0;
 }
 
+// The plan a search of (N, ld, Q, k) on one of `shards` row shards runs with, without launching anything (no GPU
+// needed): out[0..n_out) = sms, v2, nq, bn, stages, ks, grid, max_parts, S, T, W, R, n_main, Tmain, Tt, sample_m,
+// sample_gw, cap, flush (R, n_main, Tmain and Tt are 0 for the single-CTA kernel, which has no such decomposition).
+// Tests use it to prove which kernel instantiation and work decomposition a shape reaches.
+extern "C" int b200rec_debug_topk_plan(int64_t N, int64_t ld, int64_t Q, int k, int shards, long long* out, int n_out) {
+  using namespace b200;
+  if (out == nullptr || n_out < 0) return fail("topk_plan: null output");
+  TopkPlan p;
+  if (search_plan(p, N, ld, Q, k, shards)) return 1;
+  const bool v2 = p.v2 != 0;
+  const long long v[] = {num_sms(), p.v2, p.nq, p.bn, p.g.stages, p.g.ks, p.g.grid, p.g.max_parts, p.g.S, p.g.T, p.g.W,
+                         v2 ? p.g.R : 0, v2 ? p.g.n_main : 0, v2 ? p.g.Tmain : 0, v2 ? p.g.Tt : 0, p.sample_m,
+                         p.sample_gw, p.cap, flush_for(p, Q, k)};
+  for (int i = 0; i < n_out && i < (int)(sizeof(v) / sizeof(v[0])); ++i) out[i] = v[i];
+  return 0;
+}
+
 extern "C" int b200rec_debug_topk_stats(unsigned long long* out8_host, int reset) {
   using namespace b200;
   B200_CUDA_OK(cudaMemcpyFromSymbol(out8_host, g_topk_stats, sizeof(unsigned long long) * 8));
@@ -1459,8 +1488,7 @@ static int topk_dispatch(const void* catalogue, int64_t N, int64_t ld, const voi
                          void* workspace, size_t workspace_bytes, void* stream) {
   using namespace b200;
   TopkPlan p;
-  if (plan_topk(p, N, ld, Q, k, shards)) return 1;
-  if (shards > 1 && p.sample_m == 0 && plan_topk(p, N, ld, Q, k)) return 1;  // pooled density too thin for this shard
+  if (search_plan(p, N, ld, Q, k, shards)) return 1;
   p.sample_k_out = sample_k_out;
   if (workspace_bytes < p.total()) return fail("topk: workspace too small (%zu < %zu)", workspace_bytes, p.total());
   if ((exclude_indptr == nullptr) != (exclude_rows == nullptr)) return fail("topk: exclusion CSR needs both arrays");

@@ -26,6 +26,28 @@ logger = logging.getLogger("b200rec")
 FLT_MAX = float(np.finfo(np.float32).max)
 
 
+def _max_dimension(storage: str) -> int:
+    """Largest row dimension the top-K kernels have a plan for: the resident query tile holds ld = terms * pad64(d)
+    bf16 columns (terms = 3 for fp32 storage), which the library answers without a GPU."""
+    terms = 1 if storage == "bf16" else 3
+    d = 0
+    while K.topk_workspace_bytes(1, terms * (d + 64), 1, 1) > 0:
+        d += 64
+    return d
+
+
+def check_dimension(d: int, storage: str) -> None:
+    """ValueError when d-dimensional rows in this storage cannot be searched, before any row reaches the device."""
+    if d < 1:
+        raise ValueError(f"dimension must be >= 1 (got {d})")
+    if K.topk_workspace_bytes(1, (1 if storage == "bf16" else 3) * pad64(d), 1, 1) > 0:
+        return
+    msg = f"dimension {d} is too large: the largest supported d is {_max_dimension(storage)} for storage={storage!r}"
+    if storage != "bf16":
+        msg += f"; storage='bf16' lifts the limit to {_max_dimension('bf16')}"
+    raise ValueError(msg)
+
+
 class IndexBase(ABC):
     """Abstract base class for ANN indices (reference retrieval.py:16-46)."""
 
@@ -111,6 +133,7 @@ class FlatIPDeviceIndex:
     def __init__(self, d: int, storage: str = "fp32", device: Optional[torch.device] = None, row_offset: int = 0):
         if storage not in ("bf16", "fp32"):
             raise ValueError("storage must be 'bf16' or 'fp32'")
+        check_dimension(int(d), storage)
         if not torch.cuda.is_available():
             raise RuntimeError("FlatIPDeviceIndex needs a CUDA (sm_100a) device; there is no CPU search path")
         self.d = int(d)
@@ -452,6 +475,7 @@ class B200FlatIndex(IndexBase):
         self.nprobe = self.config.get("nprobe", 20)
         self.use_gpu = True
         self.storage = self.config.get("storage", "fp32")
+        check_dimension(int(self.dimension), self.storage)
         self.filter = self.config.get("filter", "post")
         if self.filter not in ("post", "exact"):
             raise ValueError(f"filter {self.filter!r}: 'post' (the reference's post-pass over the 2k best rows) or "

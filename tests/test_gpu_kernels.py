@@ -1,7 +1,12 @@
 """GPU parity tests of the low-level kernels, called through the C-ABI (ctypes) and checked against the CPU oracle."""
+import os
+import sys
+
 import numpy as np
 import pytest
 import torch
+
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 pytestmark = pytest.mark.gpu
 
@@ -123,27 +128,27 @@ def test_flat_ip_topk_ties_and_exclusion():
     assert np.array_equal(Ig.cpu().numpy(), rI)
 
 
-@pytest.mark.parametrize("sched", ["default", "0", "3"])
+@pytest.mark.parametrize("sched", ["default", "0", "3", "4"])
 @pytest.mark.parametrize("N,Q,D,k", [(300_000, 1500, 64, 20), (150_000, 4500, 64, 10)])
-def test_flat_ip_topk_work_splits_bit_exact(monkeypatch, sched, N, Q, D, k):
-    """The 2-CTA kernel's three work decompositions (time-aligned strided sweep with idle leftover units, the same with
+def test_flat_ip_topk_work_splits_bit_exact(sched, N, Q, D, k):
+    """The 2-CTA kernel's work decompositions (time-aligned strided sweep with idle leftover units, the same with
     leftover units that change supertile and hand their lists over, contiguous split) on integer data: exact scores,
-    massive ties, so the total order (score desc, row asc) must come out bit for bit.
-    Note: since round 2 the library reads its development knobs once per process, so B200REC_SCHED only forces a
-    decomposition when this is the process's first top-K call (e.g. `pytest -k work_splits`, or an xdist worker that
-    starts here); otherwise the shape picks its own.  The shape-selected paths are also covered by
-    test_flat_ip_topk_more_supertiles_than_units (contiguous split) and by bench.py's `parity_checked` at 10 M rows
-    (leftover units that change supertile)."""
+    massive ties, so the total order (score desc, row asc) must come out bit for bit.  B200REC_SCHED is applied with
+    b200rec_debug_reload_env() and the plan query proves which decomposition ran; sched=4 idles leftover units even on
+    long scans, which on these shapes is the default decomposition (tests/test_topk_plan_host.py pins the long scan)."""
     from b200rec import kernels as KR
-    if sched != "default":
-        monkeypatch.setenv("B200REC_SCHED", sched)
+    from topk_plan import decomposition, plan, topk_knobs
     rng = np.random.default_rng(N + Q)
     base = rng.integers(-3, 4, size=(N, D)).astype(np.float32)
     qry = rng.integers(-3, 4, size=(Q, D)).astype(np.float32)
     rD, rI = _oracle_topk(base, qry, k)
-    Dg, Ig = KR.flat_ip_topk(torch.from_numpy(base).cuda().to(torch.bfloat16),
-                             torch.from_numpy(qry).cuda().to(torch.bfloat16), k)
-    torch.cuda.synchronize()
+    with topk_knobs(B200REC_SCHED=None if sched == "default" else sched):
+        p = plan(N, D, Q, k)
+        split = {"default": "aligned-idle", "0": "contiguous", "3": "aligned-working", "4": "aligned-idle"}[sched]
+        assert p["v2"] == 2 and decomposition(p) == split, p
+        Dg, Ig = KR.flat_ip_topk(torch.from_numpy(base).cuda().to(torch.bfloat16),
+                                 torch.from_numpy(qry).cuda().to(torch.bfloat16), k)
+        torch.cuda.synchronize()
     assert np.array_equal(Dg.cpu().numpy(), rD)
     assert np.array_equal(Ig.cpu().numpy(), rI)
 
