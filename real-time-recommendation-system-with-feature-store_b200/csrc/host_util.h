@@ -50,4 +50,8 @@ inline int num_sms() {
 int make_tmap_bf16_2d(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t ld,
                       uint32_t box_rows);
 
+// the fused in-batch log-sum-exp plan of (B, NI, ld), for the loss plan query (inbatch_lse.cu)
+constexpr int LSE_PLAN_FIELDS = 8;
+void lse_plan_fields(int64_t B, int64_t NI, int64_t ld, long long (&v)[LSE_PLAN_FIELDS]);
+
 }  // namespace b200

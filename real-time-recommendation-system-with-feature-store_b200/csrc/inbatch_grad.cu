@@ -419,29 +419,30 @@ inbatch_grad_kernel(const __grid_constant__ CUtensorMap tm_ux, const __grid_cons
 
 // ring sizes / shared memory of the instantiation that serves (E, nprod_s, nprod_g); false when none fits
 template <int E, int NPS, int NPG>
-static bool ig_cfg_get(int& smem) {
+static bool ig_cfg_get(int& smem, int& nst) {
   smem = IgCfg<E, NPS, NPG>::SMEM;
+  nst = IgCfg<E, NPS, NPG>::NST;
   return IgCfg<E, NPS, NPG>::OK;
 }
 
-static bool ig_cfg(int E, int nps, int npg, int& smem) {
+static bool ig_cfg(int E, int nps, int npg, int& smem, int& nst) {
   if (E == 64) {
-    if (nps == 1 && npg == 1) return ig_cfg_get<64, 1, 1>(smem);
-    if (nps == 3 && npg == 3) return ig_cfg_get<64, 3, 3>(smem);
-    if (nps == 6 && npg == 3) return ig_cfg_get<64, 6, 3>(smem);
+    if (nps == 1 && npg == 1) return ig_cfg_get<64, 1, 1>(smem, nst);
+    if (nps == 3 && npg == 3) return ig_cfg_get<64, 3, 3>(smem, nst);
+    if (nps == 6 && npg == 3) return ig_cfg_get<64, 6, 3>(smem, nst);
   } else if (E == 128) {
-    if (nps == 1 && npg == 1) return ig_cfg_get<128, 1, 1>(smem);
-    if (nps == 3 && npg == 3) return ig_cfg_get<128, 3, 3>(smem);
-    if (nps == 6 && npg == 3) return ig_cfg_get<128, 6, 3>(smem);
+    if (nps == 1 && npg == 1) return ig_cfg_get<128, 1, 1>(smem, nst);
+    if (nps == 3 && npg == 3) return ig_cfg_get<128, 3, 3>(smem, nst);
+    if (nps == 6 && npg == 3) return ig_cfg_get<128, 6, 3>(smem, nst);
   }
   return false;
 }
 
-static int ig_plan(IgArgs& a, int64_t B, int64_t NI, int E, int nprod_s, int nprod_g, int& smem_bytes) {
+static int ig_plan(IgArgs& a, int64_t B, int64_t NI, int E, int nprod_s, int nprod_g, int& smem_bytes, int& nst) {
   if (E != 64 && E != 128) return fail("inbatch_grad: fused path needs E = 64 or 128 (got %d)", E);
   if (!((nprod_s == 1 && nprod_g == 1) || (nprod_s == 3 && nprod_g == 3) || (nprod_s == 6 && nprod_g == 3)))
     return fail("inbatch_grad: piece products (logits, gradient) must be (1,1), (3,3) or (6,3)");
-  if (!ig_cfg(E, nprod_s, nprod_g, smem_bytes))
+  if (!ig_cfg(E, nprod_s, nprod_g, smem_bytes, nst))
     return fail("inbatch_grad: E = %d with %d piece products does not fit the resident tile", E, nprod_s);
   // units of equal length: L = tiles of the shorter column range, capped (accumulator chains, tail balance)
   const int64_t tu = (NI + IG_BN - 1) / IG_BN, tv = (B + IG_BN - 1) / IG_BN;
@@ -484,9 +485,32 @@ using namespace b200;
 
 extern "C" int b200rec_inbatch_grad_supported(int64_t B, int64_t NI, int E, int nprod_s, int nprod_g) {
   IgArgs a;
-  int smem = 0;
+  int smem = 0, nst = 0;
   if (B <= 0 || NI <= 0 || B > INT32_MAX / 2 || NI > INT32_MAX / 2) return 0;
-  return ig_plan(a, B, NI, E, nprod_s, nprod_g, smem) == 0 ? 1 : 0;
+  return ig_plan(a, B, NI, E, nprod_s, nprod_g, smem, nst) == 0 ? 1 : 0;
+}
+
+// The plans the in-batch loss runs with, without launching anything (no GPU needed): out[0..n_out) = sms, then the
+// forward log-sum-exp of (B, NI, ld) -- nq, bn, stages, grid, S, T, W, max_parts, all 0 when the operand is too wide
+// and the forward takes the GEMM + lse_rows fallback -- then the fused backward of (B, NI, E, nprod_s, nprod_g) --
+// supported, smem, NST, units_u, splits_u, splits_v, atomic_u, atomic_v, all 0 when the backward takes the chunked
+// path.  Tests use it to prove which kernel instantiation and work split a shape reaches.
+extern "C" int b200rec_debug_loss_plan(int64_t B, int64_t NI, int64_t ld, int E, int nprod_s, int nprod_g,
+                                       long long* out, int n_out) {
+  if (out == nullptr || n_out < 0) return fail("loss_plan: null output");
+  if (B <= 0 || NI <= 0) return fail("loss_plan: empty input");
+  long long v[1 + LSE_PLAN_FIELDS + 8] = {num_sms()};
+  long long lse[LSE_PLAN_FIELDS];
+  lse_plan_fields(B, NI, ld, lse);
+  for (int i = 0; i < LSE_PLAN_FIELDS; ++i) v[1 + i] = lse[i];
+  IgArgs a;
+  int smem = 0, nst = 0;
+  if (b200rec_inbatch_grad_supported(B, NI, E, nprod_s, nprod_g) && ig_plan(a, B, NI, E, nprod_s, nprod_g, smem, nst) == 0) {
+    const long long g[8] = {1, smem, nst, a.units_u, a.side[0].splits, a.side[1].splits, a.atomic_u, a.atomic_v};
+    for (int i = 0; i < 8; ++i) v[1 + LSE_PLAN_FIELDS + i] = g[i];
+  }
+  for (int i = 0; i < n_out && i < (int)(sizeof(v) / sizeof(v[0])); ++i) out[i] = v[i];
+  return 0;
 }
 
 extern "C" int b200rec_inbatch_grad(const void* u_op, int64_t ld_u, const int32_t* u_pieces_host, const void* v_op,
@@ -504,8 +528,8 @@ extern "C" int b200rec_inbatch_grad(const void* u_op, int64_t ld_u, const int32_
   if ((ld_du & 3) || (ld_dv & 3) || (reinterpret_cast<uintptr_t>(dU) & 15) || (reinterpret_cast<uintptr_t>(dV) & 15))
     return fail("inbatch_grad: gradient rows must be 16-byte aligned");
   IgArgs a;
-  int smem = 0;
-  if (ig_plan(a, B, NI, E, nprod_s, nprod_g, smem)) return 1;
+  int smem = 0, nst = 0;
+  if (ig_plan(a, B, NI, E, nprod_s, nprod_g, smem, nst)) return 1;
   const int KB = E / 64;
   const int ps = nprod_s == 1 ? 1 : (nprod_s == 3 ? 2 : 3), pg = nprod_g == 1 ? 1 : 2;
   IgSide& su = a.side[0];

@@ -148,6 +148,18 @@ static int plan_lse(LsePlan& p, int64_t B, int64_t NI, int64_t ld) {
   return 0;
 }
 
+// plan_lse's choice for b200rec_debug_loss_plan: nq, bn, stages, grid, S, T, W, max_parts; all 0 when there is no fused
+// plan (b200rec_inbatch_lse_workspace_bytes returns 0 and the caller takes the GEMM + lse_rows fallback)
+void lse_plan_fields(int64_t B, int64_t NI, int64_t ld, long long (&v)[LSE_PLAN_FIELDS]) {
+  LsePlan p;
+  if (plan_lse(p, B, NI, ld)) {
+    for (long long& x : v) x = 0;
+    return;
+  }
+  const long long f[LSE_PLAN_FIELDS] = {p.nq, p.bn, p.g.stages, p.g.grid, p.g.S, p.g.T, p.g.W, p.g.max_parts};
+  for (int i = 0; i < LSE_PLAN_FIELDS; ++i) v[i] = f[i];
+}
+
 template <int NQ, int BN>
 static int launch_lse(const LsePlan& p, const void* U, const void* I, int64_t ld, int64_t B, int64_t NI, float inv_t,
                       float* lse, void* workspace, cudaStream_t st) {

@@ -221,7 +221,11 @@ extern "C" int b200rec_explicit_ce(const float* U, const float* P, const float* 
   if (B <= 0 || R <= 0 || E <= 0) return fail("explicit_ce: empty input");
   if (R > 4095) return fail("explicit_ce: at most 4095 negatives per sample");
   if (dU && (!dP || !dN)) return fail("explicit_ce: gradient outputs must be given together");
+  // one row of R + 1 logits per warp: above the 48 KB default (R >= 1536) the kernel has to opt in, up to 128 KB at
+  // R = 4095.  Set per launch, not once per process: the attribute belongs to the current device.
   const size_t smem = 8 * (size_t)(R + 1) * sizeof(float);
+  if (smem > 48 * 1024)
+    B200_CUDA_OK(cudaFuncSetAttribute(explicit_ce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   explicit_ce_kernel<<<warp_rows_grid(B), 256, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
       U, P, Nn, B, (int)R, E, inv_temperature, user_bias, item_bias, row_loss, grad_scale, grad_scale_dev, dU, dP, dN,
       row_dbias);
