@@ -84,6 +84,38 @@ int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, int64_t ld, 
 int b200rec_rows_to_bitmap(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, void* stream);
 int b200rec_remap_ids(const int64_t* ids, int64_t n, const int64_t* rows, int64_t n_rows, int64_t row_offset,
                       int64_t* out, void* stream);
+/* Mutable catalogue (csrc/mutate.cu; FlatIPDeviceIndex.update_rows / remove_rows / compact).  Row slots never move:
+ * the index keeps a live-row bitmap (IDSelectorBitmap layout as above, one bit per slot) and searches it as an allow
+ * bitmap once a row has been removed.
+ * b200rec_update_rows: b200rec_normalize_rows (faiss rule, normalize != 0) whose source row i is written to slot
+ * dst_rows[i] of dst_bf16 [n_slots, terms*kpad] and of dst_f32 [n_slots, ld_f32] (nullable), in place; live_bits
+ * (nullable) gets those slots' bits set in the same launch (an update revives a removed row).  dst_rows are distinct
+ * (which of two equal destinations wins is unspecified); slots outside [0, n_slots) are skipped.
+ * b200rec_clear_row_bits: clears the bits of rows[0..n) in place (b200rec_rows_to_bitmap clears the whole bitmap and
+ * sets); rows outside [0, n_bits) are ignored, duplicates are harmless.
+ * b200rec_patch_compacted: keeps a compacted filter operand (compact [n_filter, ld] bf16, row j = operand row
+ * filter_rows[j], filter_rows ascending) in step with the index after one mutation batch, in one launch.  Each of
+ * changed_rows[0..n_changed) is looked up in filter_rows; where found at j, update != 0 copies operand row r into compact
+ * row j and sets bit j of compact_bits (nullable for updates), update == 0 clears bit j (compact_bits required, the
+ * operands are then ignored).  ld (elements) is a multiple of 8.
+ * b200rec_flat_ip_topk_masked: b200rec_flat_ip_topk with any combination of the exclusion CSR, an allow bitmap
+ * (allow_bits / allow_n as in b200rec_flat_ip_topk_filtered), a remap table (remap_rows / n_remap = N: the catalogue is
+ * compacted, its row j is local row remap_rows[j], ids = remap_rows[j] + row_offset, mapped inside the select kernel) and
+ * tau_init.  Exclusion rows and allow bits index the catalogue as given (compacted rows when remap_rows is given).  A row
+ * is a candidate when it is allowed and not excluded; the sampling pass runs over allowed rows only and is skipped under
+ * exclusion lists or tau_init, as in b200rec_flat_ip_topk. */
+int b200rec_update_rows(const float* src, int64_t rows, int64_t cols, int64_t ld_src, int normalize,
+                        const int64_t* dst_rows, int64_t n_slots, float* dst_f32, int64_t ld_f32, void* dst_bf16,
+                        int64_t kpad, int terms, int side, uint32_t* live_bits, void* stream);
+int b200rec_clear_row_bits(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, void* stream);
+int b200rec_patch_compacted(const int64_t* changed_rows, int64_t n_changed, const int64_t* filter_rows, int64_t n_filter,
+                            const void* operand, int64_t ld, void* compact, uint32_t* compact_bits, int update,
+                            void* stream);
+int b200rec_flat_ip_topk_masked(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
+                                int64_t row_offset, const int64_t* exclude_indptr, const int32_t* exclude_rows,
+                                const uint32_t* allow_bits, int64_t allow_n, const int64_t* remap_rows, int64_t n_remap,
+                                const float* tau_init, float* out_scores, int64_t* out_ids, void* workspace,
+                                size_t workspace_bytes, void* stream);
 /* Sampling pass alone: out_vals [Q,k_out] = the k_out (<= k) largest group maxima (distinct sampled rows) of every
  * query, descending.  Row-sharded search exchanges these (all-gather) and starts every shard from the k-th best of the
  * union; `shards` (>= 1) says how many shards pool their samples, so each one samples 1/shards as densely.

@@ -33,6 +33,11 @@ SIGNATURES = {
     "b200rec_flat_ip_topk_filtered": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _I64, _P, _P, _P, _SZ, _P]),
     "b200rec_rows_to_bitmap": (_I, [_P, _I64, _I64, _P, _P]),
     "b200rec_remap_ids": (_I, [_P, _I64, _P, _I64, _I64, _P, _P]),
+    "b200rec_update_rows": (_I, [_P, _I64, _I64, _I64, _I, _P, _I64, _P, _I64, _P, _I64, _I, _I, _P, _P]),
+    "b200rec_clear_row_bits": (_I, [_P, _I64, _I64, _P, _P]),
+    "b200rec_patch_compacted": (_I, [_P, _I64, _P, _I64, _P, _I64, _P, _P, _I, _P]),
+    "b200rec_flat_ip_topk_masked": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _P, _P, _I64, _P, _I64, _P, _P, _P, _P,
+                                         _SZ, _P]),
     "b200rec_topk_sample": (_I, [_P, _I64, _I64, _P, _I64, _I, _I, _I, _P, _P, _SZ, _P]),
     "b200rec_topk_has_sample": (_I, [_I64, _I64, _I64, _I]),
     "b200rec_topk_pooled_kth": (_I, [_P, _I, _I64, _I, _I, _P, _P]),

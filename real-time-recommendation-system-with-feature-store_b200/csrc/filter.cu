@@ -8,11 +8,16 @@
 
 namespace b200 {
 
+// set (or, set == 0, clear) the bits of rows[0..n); rows_to_bitmap clears the bitmap first, the live-row bitmap of a
+// mutable index is edited in place (b200rec_clear_row_bits, csrc/mutate.cu)
 __global__ void __launch_bounds__(256)
-rows_to_bitmap_kernel(const int64_t* __restrict__ rows, int64_t n, int64_t n_bits, uint32_t* __restrict__ bits) {
+rows_to_bitmap_kernel(const int64_t* __restrict__ rows, int64_t n, int64_t n_bits, uint32_t* __restrict__ bits, int set) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = __ldg(rows + i);
-    if (r >= 0 && r < n_bits) atomicOr(bits + (r >> 5), 1u << (r & 31));
+    if (r >= 0 && r < n_bits) {
+      if (set) atomicOr(bits + (r >> 5), 1u << (r & 31));
+      else atomicAnd(bits + (r >> 5), ~(1u << (r & 31)));
+    }
   }
 }
 
@@ -31,6 +36,12 @@ static int grid_for(int64_t n) {
   return (int)(blocks < cap ? (blocks > 0 ? blocks : 1) : cap);
 }
 
+int launch_row_bits(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, int set, cudaStream_t st) {
+  rows_to_bitmap_kernel<<<grid_for(n), 256, 0, st>>>(rows, n, n_bits, bits, set);
+  B200_LAUNCH_OK("rows_to_bitmap_kernel");
+  return 0;
+}
+
 }  // namespace b200
 
 extern "C" int b200rec_rows_to_bitmap(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, void* stream) {
@@ -40,9 +51,7 @@ extern "C" int b200rec_rows_to_bitmap(const int64_t* rows, int64_t n, int64_t n_
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   B200_CUDA_OK(cudaMemsetAsync(bits, 0, (size_t)((n_bits + 31) / 32) * sizeof(uint32_t), st));
   if (n == 0) return 0;
-  rows_to_bitmap_kernel<<<grid_for(n), 256, 0, st>>>(rows, n, n_bits, bits);
-  B200_LAUNCH_OK("rows_to_bitmap_kernel");
-  return 0;
+  return launch_row_bits(rows, n, n_bits, bits, 1, st);
 }
 
 extern "C" int b200rec_remap_ids(const int64_t* ids, int64_t n, const int64_t* rows, int64_t n_rows, int64_t row_offset,

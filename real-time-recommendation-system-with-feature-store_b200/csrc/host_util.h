@@ -54,4 +54,11 @@ int make_tmap_bf16_2d(CUtensorMap* out, const void* base, uint64_t rows, uint64_
 constexpr int LSE_PLAN_FIELDS = 8;
 void lse_plan_fields(int64_t B, int64_t NI, int64_t ld, long long (&v)[LSE_PLAN_FIELDS]);
 
+// launchers shared across translation units: the row pass of prep.cu (dst_rows / live_bits nullable) and the row-bit
+// kernel of filter.cu (set = 1 sets, 0 clears); both validate nothing beyond what their C-ABI callers checked
+int launch_prep_rows(const float* src, int64_t rows, int64_t cols, int64_t ld_src, int normalize, int faiss_zero_rule,
+                     float* dst_f32, int64_t ld_dst, float* norms_out, void* dst_bf16, int64_t kpad, int terms, int side,
+                     const int64_t* dst_rows, int64_t n_dst, uint32_t* live_bits, cudaStream_t st);
+int launch_row_bits(const int64_t* rows, int64_t n, int64_t n_bits, uint32_t* bits, int set, cudaStream_t st);
+
 }  // namespace b200

@@ -53,17 +53,23 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
-// one warp per row
+// one warp per row.  dst_rows (nullable): source row r is written to destination row dst_rows[r] of dst_f32 / dst_bf16
+// (rows outside [0, n_dst) are skipped) and, when live_bits is given, that row's bit is set (in-place catalogue updates,
+// csrc/mutate.cu); norms_out stays indexed by the source row
 __global__ void __launch_bounds__(256)
 prep_rows_kernel(const float* __restrict__ src, int64_t rows, int64_t cols, int64_t ld_src, int normalize,
                  int faiss_zero_rule, float* __restrict__ dst_f32, int64_t ld_dst, float* __restrict__ norms_out,
-                 __nv_bfloat16* __restrict__ dst_bf16, int64_t kpad, int terms, int side) {
+                 __nv_bfloat16* __restrict__ dst_bf16, int64_t kpad, int terms, int side,
+                 const int64_t* __restrict__ dst_rows, int64_t n_dst, uint32_t* __restrict__ live_bits) {
   const int lane = threadIdx.x & 31;
   const int64_t warps_total = (int64_t)gridDim.x * (blockDim.x >> 5);
   const bool vec_ok = ((ld_src & 3) == 0) && ((reinterpret_cast<uintptr_t>(src) & 15) == 0) &&
                       ((reinterpret_cast<uintptr_t>(dst_bf16) & 15) == 0) && ((kpad & 7) == 0);
   for (int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < rows; r += warps_total) {
     const float* srow = src + r * ld_src;
+    const int64_t dr = dst_rows ? __ldg(dst_rows + r) : r;
+    if (dst_rows && (dr < 0 || dr >= n_dst)) continue;
+    if (live_bits && lane == 0) atomicOr(live_bits + (dr >> 5), 1u << (dr & 31));
     float scale = 1.0f, denom = 1.0f;
     if (normalize) {
       float ss = 0.f;
@@ -84,7 +90,7 @@ prep_rows_kernel(const float* __restrict__ src, int64_t rows, int64_t cols, int6
         if (norms_out && lane == 0) norms_out[r] = nrm;
       }
     }
-    __nv_bfloat16* drow = dst_bf16 ? dst_bf16 + r * terms * kpad : nullptr;
+    __nv_bfloat16* drow = dst_bf16 ? dst_bf16 + dr * terms * kpad : nullptr;
     if (drow && vec_ok) {
       // 8 columns per lane: two 128-bit loads, one 128-bit store per term block (2-byte stores ran at 1 TB/s)
       for (int64_t c = (int64_t)lane * 8; c < kpad; c += 256) {
@@ -101,7 +107,7 @@ prep_rows_kernel(const float* __restrict__ src, int64_t rows, int64_t cols, int6
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           if (normalize) x[j] = faiss_zero_rule ? x[j] * scale : x[j] / denom;
-          if (dst_f32 && c + j < cols) dst_f32[r * ld_dst + c + j] = x[j];
+          if (dst_f32 && c + j < cols) dst_f32[dr * ld_dst + c + j] = x[j];
           split3(x[j], p[0][j], p[1][j], p[2][j]);
         }
 #pragma unroll
@@ -123,7 +129,7 @@ prep_rows_kernel(const float* __restrict__ src, int64_t rows, int64_t cols, int6
       if (c < cols) {
         x = __ldg(srow + c);
         if (normalize) x = faiss_zero_rule ? x * scale : x / denom;
-        if (dst_f32) dst_f32[r * ld_dst + c] = x;
+        if (dst_f32) dst_f32[dr * ld_dst + c] = x;
       }
       if (drow) store_terms(drow, c, kpad, terms, side, x);
     }
@@ -178,6 +184,23 @@ static int check_terms(int terms, int side) {
   return 0;
 }
 
+// the row pass of b200rec_normalize_rows with a destination row list (b200rec_update_rows, csrc/mutate.cu)
+int launch_prep_rows(const float* src, int64_t rows, int64_t cols, int64_t ld_src, int normalize, int faiss_zero_rule,
+                     float* dst_f32, int64_t ld_dst, float* norms_out, void* dst_bf16, int64_t kpad, int terms, int side,
+                     const int64_t* dst_rows, int64_t n_dst, uint32_t* live_bits, cudaStream_t st) {
+  if (dst_bf16) {
+    if (kpad < cols || (kpad % 8)) return fail("normalize_rows: kpad must be >= cols and a multiple of 8");
+    if (check_terms(terms, side)) return 1;
+  }
+  const int64_t blocks = (rows + 7) / 8;
+  const int grid = (int)(blocks < (int64_t)num_sms() * 16 ? blocks : (int64_t)num_sms() * 16);
+  prep_rows_kernel<<<grid, 256, 0, st>>>(src, rows, cols, ld_src, normalize, faiss_zero_rule, dst_f32, ld_dst,
+                                         norms_out, reinterpret_cast<__nv_bfloat16*>(dst_bf16), kpad, terms, side,
+                                         dst_rows, n_dst, live_bits);
+  B200_LAUNCH_OK("prep_rows_kernel");
+  return 0;
+}
+
 }  // namespace b200
 
 extern "C" int b200rec_split_bf16(const float* src, int64_t rows, int64_t cols, int64_t ld_src, int transpose,
@@ -192,7 +215,7 @@ extern "C" int b200rec_split_bf16(const float* src, int64_t rows, int64_t cols, 
     const int64_t blocks = (rows + 7) / 8;
     const int grid = (int)(blocks < (int64_t)num_sms() * 16 ? blocks : (int64_t)num_sms() * 16);
     prep_rows_kernel<<<grid, 256, 0, st>>>(src, rows, cols, ld_src, 0, 0, nullptr, 0, nullptr,
-                                           reinterpret_cast<__nv_bfloat16*>(dst), kpad, terms, side);
+                                           reinterpret_cast<__nv_bfloat16*>(dst), kpad, terms, side, nullptr, 0, nullptr);
     B200_LAUNCH_OK("prep_rows_kernel");
   } else {
     dim3 grid((unsigned)((kpad + 127) / 128), (unsigned)((rows + 31) / 32));
@@ -210,15 +233,6 @@ extern "C" int b200rec_normalize_rows(const float* src, int64_t rows, int64_t co
   using namespace b200;
   if (!src) return fail("normalize_rows: null src");
   if (rows <= 0 || cols <= 0) return fail("normalize_rows: empty input");
-  if (dst_bf16) {
-    if (kpad < cols || (kpad % 8)) return fail("normalize_rows: kpad must be >= cols and a multiple of 8");
-    if (check_terms(terms, side)) return 1;
-  }
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const int64_t blocks = (rows + 7) / 8;
-  const int grid = (int)(blocks < (int64_t)num_sms() * 16 ? blocks : (int64_t)num_sms() * 16);
-  prep_rows_kernel<<<grid, 256, 0, st>>>(src, rows, cols, ld_src, normalize, faiss_zero_rule, dst_f32, ld_dst,
-                                         norms_out, reinterpret_cast<__nv_bfloat16*>(dst_bf16), kpad, terms, side);
-  B200_LAUNCH_OK("prep_rows_kernel");
-  return 0;
+  return launch_prep_rows(src, rows, cols, ld_src, normalize, faiss_zero_rule, dst_f32, ld_dst, norms_out, dst_bf16,
+                          kpad, terms, side, nullptr, 0, nullptr, reinterpret_cast<cudaStream_t>(stream));
 }

@@ -1530,6 +1530,20 @@ extern "C" int b200rec_flat_ip_topk_filtered(const void* catalogue, int64_t N, i
                        nullptr, out_scores, out_ids, nullptr, k, 1, nullptr, nullptr, workspace, workspace_bytes, stream);
 }
 
+extern "C" int b200rec_flat_ip_topk_masked(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                           int k, int64_t row_offset, const int64_t* exclude_indptr,
+                                           const int32_t* exclude_rows, const uint32_t* allow_bits, int64_t allow_n,
+                                           const int64_t* remap_rows, int64_t n_remap, const float* tau_init,
+                                           float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                                           void* stream) {
+  if (!catalogue || !queries || !out_scores || !out_ids || !workspace) return b200::fail("topk_masked: null pointer");
+  if (allow_bits != nullptr && allow_n < 0) return b200::fail("topk_masked: allow_n must be >= 0");
+  if (remap_rows != nullptr && n_remap != N) return b200::fail("topk_masked: n_remap must equal N (one row per catalogue row)");
+  const int64_t an = allow_bits != nullptr ? (allow_n < N ? allow_n : N) : 0;
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, exclude_indptr, exclude_rows, allow_bits, an, tau_init,
+                       out_scores, out_ids, nullptr, k, 1, nullptr, remap_rows, workspace, workspace_bytes, stream);
+}
+
 extern "C" int b200rec_topk_sample(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
                                    int k_out, int shards, float* out_vals, void* workspace, size_t workspace_bytes,
                                    void* stream) {

@@ -143,6 +143,63 @@ def remap_ids(ids: torch.Tensor, rows: torch.Tensor, row_offset: int = 0) -> tor
     return ids
 
 
+def flat_ip_topk_masked(catalogue: torch.Tensor, queries: torch.Tensor, k: int, row_offset: int = 0,
+                        exclude_indptr: Optional[torch.Tensor] = None, exclude_rows: Optional[torch.Tensor] = None,
+                        allow_bits: Optional[torch.Tensor] = None, allow_n: int = 0,
+                        remap_rows: Optional[torch.Tensor] = None, tau_init: Optional[torch.Tensor] = None,
+                        workspace: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """flat_ip_topk with any combination of exclusion CSR, allow bitmap (over `catalogue` rows, rows >= allow_n out),
+    remap table (int64 [N]: `catalogue` is compacted, its row j is reported as remap_rows[j] + row_offset) and tau_init."""
+    assert catalogue.dtype == BF16 and queries.dtype == BF16
+    assert catalogue.stride(1) == 1 and queries.stride(1) == 1 and catalogue.stride(0) == queries.stride(0)
+    assert allow_bits is None or allow_bits.dtype == torch.int32
+    assert remap_rows is None or (remap_rows.dtype == torch.int64 and remap_rows.numel() == catalogue.shape[0])
+    n, ld = catalogue.shape[0], catalogue.stride(0)
+    q = queries.shape[0]
+    need = topk_workspace_bytes(n, ld, q, k)
+    if need == 0:
+        raise RuntimeError(f"b200rec flat_ip_topk_masked: {N.last_error()}")
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty((need,), dtype=torch.uint8, device=catalogue.device)
+    scores = torch.empty((q, k), dtype=torch.float32, device=catalogue.device)
+    ids = torch.empty((q, k), dtype=torch.int64, device=catalogue.device)
+    N.check(N.lib().b200rec_flat_ip_topk_masked(N.ptr(catalogue), n, ld, N.ptr(queries), q, k, row_offset,
+                                                N.ptr(exclude_indptr), N.ptr(exclude_rows), N.ptr(allow_bits), allow_n,
+                                                N.ptr(remap_rows), 0 if remap_rows is None else remap_rows.numel(),
+                                                N.ptr(tau_init), N.ptr(scores), N.ptr(ids), N.ptr(workspace),
+                                                workspace.numel(), N.stream()), "flat_ip_topk_masked")
+    return scores, ids
+
+
+def update_rows(x: torch.Tensor, dst_rows: torch.Tensor, operand: torch.Tensor, kpad: int, terms: int,
+                f32: Optional[torch.Tensor] = None, live_bits: Optional[torch.Tensor] = None,
+                normalize: bool = False) -> None:
+    """Row i of x (fp32 [n, d]) -> slot dst_rows[i] (int64, distinct) of the catalogue operand [slots, terms*kpad] (right
+    operand pattern) and of the fp32 rows f32 [slots, d]; sets the slots' bits in live_bits.  normalize: faiss rule."""
+    assert x.dtype == torch.float32 and x.stride(1) == 1 and dst_rows.dtype == torch.int64 and dst_rows.is_contiguous()
+    assert operand.dtype == BF16 and operand.is_contiguous() and dst_rows.numel() == x.shape[0]
+    N.check(N.lib().b200rec_update_rows(N.ptr(x), x.shape[0], x.shape[1], x.stride(0), int(normalize), N.ptr(dst_rows),
+                                        operand.shape[0], N.ptr(f32), 0 if f32 is None else f32.stride(0), N.ptr(operand),
+                                        kpad, terms, 1, N.ptr(live_bits), N.stream()), "update_rows")
+
+
+def clear_row_bits(rows: torch.Tensor, bits: torch.Tensor, n_bits: int) -> None:
+    """Clear the bits of `rows` (int64) in the int32 bitmap `bits`, in place."""
+    assert rows.dtype == torch.int64 and rows.is_contiguous() and bits.dtype == torch.int32
+    N.check(N.lib().b200rec_clear_row_bits(N.ptr(rows), rows.numel(), n_bits, N.ptr(bits), N.stream()), "clear_row_bits")
+
+
+def patch_compacted(changed: torch.Tensor, filter_rows: torch.Tensor, operand: Optional[torch.Tensor],
+                    compact: Optional[torch.Tensor], compact_bits: Optional[torch.Tensor], update: bool) -> None:
+    """Bring a compacted filter operand up to date after one mutation batch (`changed` int64 index rows): update copies the
+    changed rows the filter holds from `operand` and sets their compact bits, removal clears them."""
+    assert changed.dtype == torch.int64 and filter_rows.dtype == torch.int64
+    ld = 0 if operand is None else operand.stride(0)
+    N.check(N.lib().b200rec_patch_compacted(N.ptr(changed), changed.numel(), N.ptr(filter_rows), filter_rows.numel(),
+                                            N.ptr(operand), ld, N.ptr(compact), N.ptr(compact_bits), int(update),
+                                            N.stream()), "patch_compacted")
+
+
 def topk_pooled_kth(vals: torch.Tensor, k: int) -> torch.Tensor:
     """vals [parts, Q, k_in] fp32 (contiguous) -> [Q]: k-th largest of each query's parts*k_in pooled sample maxima."""
     assert vals.dim() == 3 and vals.is_contiguous() and vals.dtype == torch.float32

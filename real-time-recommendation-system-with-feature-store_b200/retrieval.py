@@ -11,7 +11,9 @@ from __future__ import annotations
 import logging
 import pickle
 import struct
+import heapq
 import time
+import weakref
 from abc import ABC, abstractmethod
 from pathlib import Path
 from typing import Any, Dict, List, Optional, Tuple
@@ -81,15 +83,23 @@ class RowFilter:
     `compacted()` is the catalogue operand restricted to the allowed rows ([n_allowed, ld] bf16, n_allowed * ld * 2
     bytes: 2.56 GB for an all-allowed filter over 10 M x 128 rows), gathered on first use and kept with the filter, so a
     filter reused across requests ("in stock") pays the gather once; flat-index rows never move, so `add` does not
-    invalidate it."""
+    invalidate it.
+
+    On a mutated index the filter keeps its row set and answers over (filter rows AND live rows) with the current row
+    contents: `update_rows` / `remove_rows` patch the compacted copy in place (and its live bitmap in compact-row space,
+    `_compact_bits`), the bitmap path ANDs `bits` with the index's live bits once per mutation epoch.  `compact()`
+    renumbers the rows, after which the filter is rejected (ValueError)."""
 
     def __init__(self, index: "FlatIPDeviceIndex", rows: np.ndarray):
         self.index = index
         self.n_bits = index.ntotal
         self.n_allowed = int(rows.size)
+        self.generation = index._generation
         self.rows = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.int64)).to(index.device)
         self.bits = K.rows_to_bitmap(self.rows, max(self.n_bits, 1))
         self._compact: Optional[torch.Tensor] = None
+        self._compact_bits: Optional[torch.Tensor] = None     # compact-row live bits, once the index has removed rows
+        self._live_and: Optional[Tuple[int, torch.Tensor]] = None   # (mutation epoch, bits AND live bits)
 
     @property
     def fraction(self) -> float:
@@ -104,7 +114,21 @@ class RowFilter:
             # bf16 rows viewed as fp32 words (ld * 2 bytes is a multiple of 128 B): the feed's row gather does the copy
             K.gather_rows(ix._cat[: self.n_bits].view(torch.float32), self.rows, err, out=out.view(torch.float32))
             self._compact = out
+            if ix._n_dead > 0:                   # rows of the filter removed before the gather stay in, bit cleared
+                r = self.rows                    # compact bit j = live bit of row rows[j], packed on the device
+                bit = (ix._live_bits[r >> 5] >> (r & 31)) & 1
+                b = torch.nn.functional.pad(bit, (0, (-self.n_allowed) % 32)).view(-1, 32)
+                words = (b << torch.arange(32, device=ix.device)).sum(1)
+                self._compact_bits = torch.where(words >= 1 << 31, words - (1 << 32), words).to(torch.int32)
+            ix._compact_filters.add(self)        # patched by every later mutation of the index
         return self._compact
+
+    def live_bits(self) -> torch.Tensor:
+        """`bits` AND the index's live-row bits (bitmap path on an index with removed rows), cached per mutation epoch."""
+        ix = self.index
+        if self._live_and is None or self._live_and[0] != ix._epoch:
+            self._live_and = (ix._epoch, torch.bitwise_and(self.bits, ix._live_bits[: self.bits.numel()]))
+        return self._live_and[1]
 
 
 class FlatIPDeviceIndex:
@@ -116,6 +140,16 @@ class FlatIPDeviceIndex:
     candidates with 3 piece products (|err| <= ~1e-5 * |q||x|), `b200rec_rescore_fp32` recomputes those candidates'
     inner products with fp32 FMAs from the fp32 rows and a final select orders them (score desc, row asc): scores are
     fp32-exact (~1e-7), ids differ from an fp32 CPU search only where fp32 summation order itself decides.
+
+    Mutable catalogue: `update_rows(rows, x)` overwrites row slots in place, `remove_rows(rows)` tombstones them and
+    `compact()` drops the removed slots (the only operation that renumbers rows).  `ntotal` counts row slots, `n_live`
+    the rows a search can return; every search path returns live rows only.  Until the first removal the index runs
+    exactly the unmutated code; after it, a live-row bitmap (one bit per slot, kept on the device and mirrored on the
+    host) is tested inside the fused kernel.  Mutations are enqueued on the caller's current CUDA stream: a search issued
+    on that stream after a mutation call has returned sees the mutation (`search` / `search_stream` search on the current
+    stream, so batches submitted after an update see it).  The row-sharded steps (`sample_device`, `sample_fanout`,
+    `search_fanout`, `sample_filtered`, `search_filtered_shard`) do not read the live bitmap and refuse an index with
+    removed rows.
     """
 
     @staticmethod
@@ -148,6 +182,15 @@ class FlatIPDeviceIndex:
         self._cat = torch.empty((0, self.ld), dtype=torch.bfloat16, device=self.device)
         self._f32 = torch.empty((0, self.d), dtype=torch.float32, device=self.device) if storage == "fp32" else None
         self._ws: Optional[torch.Tensor] = None
+        # mutation state: live bits allocated on the first removal (all ones over the reserved slots, so `add` never
+        # touches them), host mirror of the same bits, removed-slot count, epoch (bumped by every mutation) and
+        # generation (bumped by compact(): row filters of an older generation are rejected)
+        self._live_bits: Optional[torch.Tensor] = None
+        self._live_host: Optional[np.ndarray] = None
+        self._n_dead = 0
+        self._epoch = 0
+        self._generation = 0
+        self._compact_filters: "weakref.WeakSet[RowFilter]" = weakref.WeakSet()
 
     # ------------------------------------------------------------------ rows
     def _reserve(self, n: int) -> None:
@@ -161,6 +204,13 @@ class FlatIPDeviceIndex:
             nf = torch.empty((cap, self.d), dtype=torch.float32, device=self.device)
             nf[: self.ntotal] = self._f32[: self.ntotal]
             self._f32 = nf
+        if self._live_bits is not None:         # new slots are live
+            nb = torch.full(((cap + 31) // 32,), -1, dtype=torch.int32, device=self.device)
+            nb[: self._live_bits.numel()] = self._live_bits
+            self._live_bits = nb
+            nh = np.ones(cap, dtype=bool)
+            nh[: self._live_host.size] = self._live_host
+            self._live_host = nh
 
     def add(self, x, normalize: bool = False) -> None:
         """Append rows (np.ndarray or torch tensor [n, d], any float dtype).  normalize=True applies faiss.normalize_L2."""
@@ -183,7 +233,9 @@ class FlatIPDeviceIndex:
         self.ntotal += n
 
     def add_bf16_rows(self, rows: torch.Tensor) -> None:
-        """Append rows that already are bf16 operands [n, ld] on the device (bulk loaders; storage 'bf16' only)."""
+        """Append rows that already are bf16 operands [n, ld] on the device (bulk loaders; storage 'bf16' only).  Into an
+        empty index a contiguous tensor is taken over without a copy: the index then owns it, and `update_rows` writes
+        into that tensor (until a later `add` or `compact()` moves the rows to storage of the index's own)."""
         assert self.storage == "bf16" and rows.dtype == torch.bfloat16 and rows.shape[1] == self.ld
         if self.ntotal == 0 and rows.is_contiguous() and rows.device == self.device:
             self._cat = rows
@@ -191,6 +243,125 @@ class FlatIPDeviceIndex:
             self._reserve(self.ntotal + rows.shape[0])
             self._cat[self.ntotal: self.ntotal + rows.shape[0]] = rows
         self.ntotal += rows.shape[0]
+
+    # ------------------------------------------------------------------ mutation
+    @property
+    def n_live(self) -> int:
+        """Rows a search can return: ntotal minus the removed slots."""
+        return self.ntotal - self._n_dead
+
+    def _check_rows(self, rows, what: str) -> np.ndarray:
+        """Host validation of a row list (before anything reaches the device): 1-D integers in [0, ntotal)."""
+        r = np.asarray(rows.detach().cpu() if torch.is_tensor(rows) else rows)
+        if r.ndim != 1:
+            raise ValueError(f"{what}: rows must be a 1-D integer array (got shape {r.shape})")
+        if r.size == 0:
+            return np.zeros(0, dtype=np.int64)
+        if not np.issubdtype(r.dtype, np.integer):
+            raise ValueError(f"{what}: rows must be an integer array (got {r.dtype})")
+        r = r.astype(np.int64, copy=False)
+        bad = (r < 0) | (r >= self.ntotal)
+        if bad.any():
+            raise ValueError(f"{what}: row {int(r[bad][0])} is outside [0, ntotal = {self.ntotal})")
+        return r
+
+    def _ensure_live(self) -> None:
+        if self._live_bits is None:
+            cap = self._cat.shape[0]
+            self._live_bits = torch.full(((cap + 31) // 32,), -1, dtype=torch.int32, device=self.device)
+            self._live_host = np.ones(cap, dtype=bool)
+
+    def _patch_filters(self, rows_dev: torch.Tensor, update: bool) -> None:
+        """One patch launch per cached compacted filter: copy updated rows in / set or clear their compact live bits."""
+        for f in list(self._compact_filters):
+            if f._compact is None or f.n_allowed == 0 or f.generation != self._generation:
+                continue
+            if update:
+                K.patch_compacted(rows_dev, f.rows, self._cat, f._compact, f._compact_bits, True)
+            else:
+                if f._compact_bits is None:
+                    f._compact_bits = torch.full(((f.n_allowed + 31) // 32,), -1, dtype=torch.int32, device=self.device)
+                K.patch_compacted(rows_dev, f.rows, None, None, f._compact_bits, False)
+
+    def update_rows(self, rows, x, normalize: bool = False) -> None:
+        """Overwrite row slots in place: x[i] (np.ndarray or torch tensor [n, d], any float dtype) goes to slot rows[i]
+        (the bf16 operand and, for storage 'fp32', the fp32 rows); normalize=True applies faiss.normalize_L2 as `add`
+        does.  A removed slot is revived.  Duplicate rows: the last occurrence wins.  ValueError (before any device
+        work) for rows outside [0, ntotal), non-integer rows or a shape mismatch."""
+        r = self._check_rows(rows, "update_rows")
+        xt = torch.as_tensor(x)
+        if xt.dim() != 2 or xt.shape[1] != self.d or xt.shape[0] != r.size:
+            raise ValueError(f"update_rows: expected [{r.size}, {self.d}] rows, got {tuple(xt.shape)}")
+        if r.size == 0:
+            return
+        u, first_rev = np.unique(r[::-1], return_index=True)     # ascending distinct rows, last occurrence of each
+        pos = r.size - 1 - first_rev
+        if not np.array_equal(pos, np.arange(r.size)):
+            xt = xt[torch.from_numpy(pos).to(xt.device)]
+        rows_dev = torch.from_numpy(u).to(self.device, non_blocking=True)
+        n, step = u.size, 1 << 20
+        for s in range(0, n, step):
+            chunk = xt[s:s + step].to(self.device, dtype=torch.float32, non_blocking=True).contiguous()
+            K.update_rows(chunk, rows_dev[s:s + chunk.shape[0]], self._cat, self.kpad, self.terms, self._f32,
+                          self._live_bits, normalize)
+        if self._live_host is not None:
+            self._n_dead -= int(np.count_nonzero(~self._live_host[u]))
+            self._live_host[u] = True
+        self._epoch += 1
+        self._patch_filters(rows_dev, update=True)
+
+    def remove_rows(self, rows) -> int:
+        """Tombstone row slots (they stay in place until `compact()`); returns how many of them were live.  Removed
+        and duplicate rows are harmless; ValueError for rows outside [0, ntotal) or non-integer rows."""
+        u = np.unique(self._check_rows(rows, "remove_rows"))
+        if u.size == 0:
+            return 0
+        self._ensure_live()
+        gone = u[self._live_host[u]]
+        if gone.size == 0:
+            return 0
+        self._live_host[gone] = False
+        self._n_dead += int(gone.size)
+        self._epoch += 1
+        rows_dev = torch.from_numpy(gone).to(self.device, non_blocking=True)
+        K.clear_row_bits(rows_dev, self._live_bits, self.ntotal)
+        self._patch_filters(rows_dev, update=False)
+        return int(gone.size)
+
+    def compact(self) -> np.ndarray:
+        """Drop the removed slots (the live rows keep their order): returns the old -> new row map (int64 [old ntotal],
+        -1 for removed rows).  Every RowFilter built before is rejected afterwards."""
+        n = self.ntotal
+        keep = np.flatnonzero(self._live_host[:n]) if self._live_host is not None else np.arange(n, dtype=np.int64)
+        remap = np.full(n, -1, dtype=np.int64)
+        remap[keep] = np.arange(keep.size, dtype=np.int64)
+        if keep.size < n:
+            idx = torch.from_numpy(keep).to(self.device)
+            err = torch.zeros((1,), dtype=torch.int32, device=self.device)
+            new = torch.empty((keep.size, self.ld), dtype=torch.bfloat16, device=self.device)
+            nf = torch.empty((keep.size, self.d), dtype=torch.float32, device=self.device) if self._f32 is not None else None
+            if keep.size:
+                K.gather_rows(self._cat[:n].view(torch.float32), idx, err, out=new.view(torch.float32))
+                if nf is not None:
+                    K.gather_rows(self._f32[:n], idx, err, out=nf)
+            self._cat, self._f32 = new, nf
+            self.ntotal = int(keep.size)
+        self._live_bits, self._live_host, self._n_dead = None, None, 0
+        self._epoch += 1
+        self._generation += 1
+        self._compact_filters = weakref.WeakSet()
+        return remap
+
+    def _require_all_live(self, what: str) -> None:
+        if self._n_dead:
+            raise ValueError(f"{what}: the index has {self._n_dead} removed rows and row-sharded search does not read "
+                             "the live-row bitmap; compact() it first")
+
+    def _check_filter(self, sel: RowFilter) -> None:
+        if sel.index is not self:
+            raise ValueError("the row filter was built for another index")
+        if sel.generation != self._generation:
+            raise ValueError("the row filter was built before compact() renumbered the rows; build it again")
 
     def reconstruct_n(self, i0: int = 0, n: Optional[int] = None) -> np.ndarray:
         n = self.ntotal - i0 if n is None else n
@@ -226,14 +397,17 @@ class FlatIPDeviceIndex:
 
     def sample_device(self, q_op: torch.Tensor, k: int, k_out: Optional[int] = None, shards: int = 1) -> torch.Tensor:
         """Sampling pass only: the k_out largest group maxima per query [nq, k_out] (exchanged between row shards)."""
+        self._require_all_live("sample_device")
         return K.topk_sample(self._cat[: self.ntotal], q_op, k, self._workspace(q_op.shape[0], k), k_out, shards)
 
     def sample_fanout(self, q_op: torch.Tensor, k: int, k_out: int, shards: int, dst_vals) -> None:
         """Sampling pass whose [nq, k_out] maxima are stored to every address in dst_vals (peer gather buffers)."""
+        self._require_all_live("sample_fanout")
         K.topk_sample_fanout(self._cat[: self.ntotal], q_op, k, k_out, shards, dst_vals, self._workspace(q_op.shape[0], k))
 
     def search_fanout(self, q_op: torch.Tensor, k: int, tau_init, dst_scores, dst_ids) -> None:
         """Local top-k (global row ids) stored to every (dst_scores[d], dst_ids[d]) address (peer gather buffers)."""
+        self._require_all_live("search_fanout")
         K.flat_ip_topk_fanout(self._cat[: self.ntotal], q_op, k, self.row_offset, tau_init, dst_scores, dst_ids,
                               self._workspace(q_op.shape[0], k))
 
@@ -264,8 +438,7 @@ class FlatIPDeviceIndex:
         if self.storage != "bf16":
             raise ValueError("row-sharded filtered search needs bf16 storage (an fp32-storage shard re-scores its "
                              "candidates from fp32 rows, which the sharded exchange does not carry)")
-        if sel.index is not self:
-            raise ValueError("the row filter was built for another index")
+        self._check_filter(sel)
         if sel.n_allowed == 0:
             return None, sel.bits, 0, None
         if compact is None:
@@ -279,6 +452,7 @@ class FlatIPDeviceIndex:
         """Sampling pass of a filtered row-sharded search: the k_out best group maxima per query over the allowed rows
         only, sampled for `shards` pooled shards; -FLT_MAX rows when this shard has no allowed row or no sampling pass
         for the shape.  Returned [nq, k_out], or stored to every address in `dst` (peer gather buffers)."""
+        self._require_all_live("sample_filtered")
         cat, bits, allow_n, _ = self._shard_operand(sel, compact)
         ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
         return K.topk_sample_filtered(cat, q_op, k, k_out, shards, bits, allow_n, ws, dst)
@@ -289,6 +463,7 @@ class FlatIPDeviceIndex:
         allowed score, or None), global row ids (row_offset added, compact ids mapped back inside the select kernel),
         -1 / -FLT_MAX padding.  Returns (D, I) (written into `out` when given), or stores the rows to every
         (dst[0][d], dst[1][d]) address and returns None."""
+        self._require_all_live("search_filtered_shard")
         cat, bits, allow_n, remap = self._shard_operand(sel, compact)
         ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
         if dst is not None:
@@ -311,15 +486,14 @@ class FlatIPDeviceIndex:
                 raise ValueError("a row filter cannot be combined with per-query exclusion lists")
             if tau_init is not None:
                 raise ValueError("a row filter cannot be combined with tau_init (row-sharded search)")
-            if sel.index is not self:
-                raise ValueError("the row filter was built for another index")
+            self._check_filter(sel)
             d, i = self._search_filtered(q_op, k, sel, sel.fraction < self.FILTER_COMPACT_BELOW)
             if out is not None:
                 out[0].copy_(d)
                 out[1].copy_(i)
                 return out
             return d, i
-        if self.ntotal == 0:
+        if self.ntotal == 0 or self._n_dead == self.ntotal:
             if out is not None:
                 out[0].fill_(-FLT_MAX)
                 out[1].fill_(-1)
@@ -327,6 +501,19 @@ class FlatIPDeviceIndex:
             return (torch.full((nq, k), -FLT_MAX, dtype=torch.float32, device=self.device),
                     torch.full((nq, k), -1, dtype=torch.int64, device=self.device))
         q32 = getattr(q_op, "_b200_f32", None) if self._f32 is not None else None
+        if self._n_dead > 0:                     # removed rows: the live bitmap as an allow bitmap, one path
+            kk = k if q32 is None else min(k + self.rescore_margin(k), max(k, min(self.ntotal, 2048)))
+            d, i = K.flat_ip_topk_masked(self._cat[: self.ntotal], q_op, kk, self.row_offset, exclude_indptr,
+                                         exclude_rows, self._live_bits, self.ntotal, None,
+                                         tau_init if q32 is None else None, self._workspace(nq, kk))
+            if q32 is not None:
+                exact = K.rescore_fp32(q32, self._f32[: self.ntotal], i, self.row_offset)
+                d, i = K.topk_merge(exact.unsqueeze(0), i.unsqueeze(0), k)
+            if out is not None:
+                out[0].copy_(d)
+                out[1].copy_(i)
+                return out
+            return d, i
         if q32 is None:
             return K.flat_ip_topk(self._cat[: self.ntotal], q_op, k, self.row_offset, exclude_indptr, exclude_rows,
                                   self._workspace(nq, k), tau_init, out)
@@ -353,10 +540,16 @@ class FlatIPDeviceIndex:
         kk = k if q32 is None else min(k + self.rescore_margin(k), max(k, min(self.ntotal, 2048)))
         if compact:
             cat = sel.compacted()
-            d, i = K.flat_ip_topk(cat, q_op, kk, 0, workspace=self._workspace(nq, kk, cat.shape[0]))
-            K.remap_ids(i, sel.rows, self.row_offset)
+            if self._n_dead > 0 and sel._compact_bits is not None:   # compact live bits + remap in the same search
+                d, i = K.flat_ip_topk_masked(cat, q_op, kk, self.row_offset, allow_bits=sel._compact_bits,
+                                             allow_n=sel.n_allowed, remap_rows=sel.rows,
+                                             workspace=self._workspace(nq, kk, cat.shape[0]))
+            else:
+                d, i = K.flat_ip_topk(cat, q_op, kk, 0, workspace=self._workspace(nq, kk, cat.shape[0]))
+                K.remap_ids(i, sel.rows, self.row_offset)
         else:
-            d, i = K.flat_ip_topk_filtered(self._cat[: self.ntotal], q_op, kk, sel.bits, sel.n_bits, self.row_offset,
+            bits = sel.live_bits() if self._n_dead > 0 else sel.bits
+            d, i = K.flat_ip_topk_filtered(self._cat[: self.ntotal], q_op, kk, bits, sel.n_bits, self.row_offset,
                                            self._workspace(nq, kk))
         if q32 is None:
             return d, i
@@ -465,7 +658,15 @@ class HostPipeline:
 
 
 class B200FlatIndex(IndexBase):
-    """`FaissIndex` on the exact Flat / inner-product branch (reference retrieval.py:49-329), B200-resident."""
+    """`FaissIndex` on the exact Flat / inner-product branch (reference retrieval.py:49-329), B200-resident.
+
+    config "updates": "warn" (default) keeps the reference's behaviour: `add` appends a row even for an id that is already
+    indexed, `update` / `remove` only log the reference's warnings.  "in_place" makes the catalogue mutable: `add` and
+    `update` are the same upsert (known ids are overwritten in place, new ids fill removed slots lowest first and then
+    append, the last occurrence of a repeated id wins), `remove(ids)` tombstones the rows of known ids, and searches
+    return live items only, so a streaming `RetrievalEngine.update_index` never returns an item twice.  `current_size`
+    then counts live items, `id_map` / `reverse_id_map` hold live rows only, `save` writes the live rows renumbered
+    densely and `compact()` drops removed slots."""
 
     def __init__(self, config: Optional[Dict[str, Any]] = None):
         self.config = config or {}
@@ -476,6 +677,10 @@ class B200FlatIndex(IndexBase):
         self.use_gpu = True
         self.storage = self.config.get("storage", "fp32")
         check_dimension(int(self.dimension), self.storage)
+        self.updates = self.config.get("updates", "warn")
+        if self.updates not in ("warn", "in_place"):
+            raise ValueError(f"updates {self.updates!r}: 'warn' (the reference: add appends, update / remove only warn) "
+                             "or 'in_place' (upsert / remove on the live catalogue)")
         self.filter = self.config.get("filter", "post")
         if self.filter not in ("post", "exact"):
             raise ValueError(f"filter {self.filter!r}: 'post' (the reference's post-pass over the 2k best rows) or "
@@ -487,6 +692,7 @@ class B200FlatIndex(IndexBase):
         self.id_map: Dict[int, str] = {}
         self.reverse_id_map: Dict[str, int] = {}
         self.current_size = 0
+        self._free: List[int] = []              # "in_place": removed slots, a min-heap (reused lowest first)
 
     def build(self, embeddings: np.ndarray, ids: List[str]):
         n_items = len(embeddings)
@@ -504,17 +710,32 @@ class B200FlatIndex(IndexBase):
             self.id_map[i] = item_id
             self.reverse_id_map[item_id] = i
         self.current_size = n_items
+        self._free = []
+        if self.updates == "in_place":           # a repeated id keeps its last row; the other rows are removed
+            self._drop_unmapped_rows()
         logger.info("Index built in %.2f seconds", time.time() - start)
+
+    def _n_rows(self) -> int:
+        """Row slots the row -> id array spans: every row of the device index under "in_place", else current_size."""
+        return self.index.ntotal if self.updates == "in_place" else self.current_size
 
     def _names(self) -> np.ndarray:
         """Row -> item id as one object array (the reference walks nq x k dict lookups in Python, retrieval.py:177-195)."""
         arr = getattr(self, "_id_array", None)
-        if arr is None or len(arr) != self.current_size:
-            arr = np.empty(self.current_size, dtype=object)
-            arr[:] = [self.id_map.get(i) for i in range(self.current_size)]
+        n = self._n_rows()
+        if arr is None or len(arr) != n:
+            arr = np.empty(n, dtype=object)
+            arr[:] = [self.id_map.get(i) for i in range(n)]
             self._id_array = arr
-            self._mapped = np.fromiter((x is not None for x in arr), dtype=bool, count=self.current_size)
+            self._mapped = np.fromiter((x is not None for x in arr), dtype=bool, count=n)
         return arr
+
+    def _set_name(self, row: int, item_id: Optional[str]) -> None:
+        """Keep the cached row -> id array in step with one in-place change (it is rebuilt when rows were appended)."""
+        arr = getattr(self, "_id_array", None)
+        if arr is not None and row < len(arr):
+            arr[row] = item_id
+            self._mapped[row] = item_id is not None
 
     def search(self, query_embeddings: np.ndarray, k: int = 10,
                filter_ids: Optional[List[str]] = None) -> Tuple[List[List[str]], List[List[float]]]:
@@ -529,6 +750,8 @@ class B200FlatIndex(IndexBase):
         if len(query_embeddings.shape) == 1:
             query_embeddings = query_embeddings.reshape(1, -1)
         exact = filter_ids is not None and self.filter == "exact"
+        if self.updates == "in_place" and self.current_size == 0:      # every item removed
+            return [[] for _ in range(len(query_embeddings))], [[] for _ in range(len(query_embeddings))]
         if exact:
             rows = np.fromiter((self.reverse_id_map[x] for x in set(filter_ids) if x in self.reverse_id_map), np.int64)
             distances, indices = self.index.search(query_embeddings, k, normalize=(self.metric == "cosine"),
@@ -539,7 +762,7 @@ class B200FlatIndex(IndexBase):
         if self.current_size == 0:
             return [[] for _ in range(len(indices))], [[] for _ in range(len(indices))]
         names = self._names()
-        keep = (indices >= 0) & (indices < self.current_size)
+        keep = (indices >= 0) & (indices < self._n_rows())
         safe = np.where(keep, indices, 0)
         keep &= self._mapped[safe]
         picked = names[safe]
@@ -556,6 +779,9 @@ class B200FlatIndex(IndexBase):
     def add(self, embeddings: np.ndarray, ids: List[str]):
         if self.index is None:
             raise ValueError("Index not built yet")
+        if self.updates == "in_place":
+            self._upsert(embeddings, ids)
+            return
         embeddings = np.asarray(embeddings).astype(np.float32)
         self.index.add(embeddings, normalize=(self.metric == "cosine"))
         for i, item_id in enumerate(ids):
@@ -566,21 +792,114 @@ class B200FlatIndex(IndexBase):
         logger.info("Added %d items to index. Total size: %d", len(embeddings), self.current_size)
 
     def update(self, embeddings: np.ndarray, ids: List[str]):
+        if self.updates == "in_place":
+            if self.index is None:
+                raise ValueError("Index not built yet")
+            self._upsert(embeddings, ids)
+            return
         logger.warning("Flat indices do not support in-place updates. Consider periodic rebuilds.")
 
     def remove(self, ids: List[str]):
-        logger.warning("Flat indices do not support removal. Consider periodic rebuilds.")
+        """"in_place": tombstone the rows of the known ids (unknown ids are ignored) and return how many were removed."""
+        if self.updates != "in_place":
+            logger.warning("Flat indices do not support removal. Consider periodic rebuilds.")
+            return
+        if self.index is None:
+            raise ValueError("Index not built yet")
+        rows = []
+        for item_id in dict.fromkeys(ids):
+            row = self.reverse_id_map.pop(item_id, None)
+            if row is not None:
+                del self.id_map[row]
+                self._set_name(row, None)
+                heapq.heappush(self._free, row)
+                rows.append(row)
+        if rows:
+            self.index.remove_rows(np.asarray(rows, dtype=np.int64))
+        self.current_size = len(self.reverse_id_map)
+        return len(rows)
+
+    def _upsert(self, embeddings, ids: List[str]) -> None:
+        """"in_place" add / update: known ids overwrite their rows, new ids take removed slots (lowest first), then
+        append; the last occurrence of a repeated id wins."""
+        embeddings = np.asarray(embeddings).astype(np.float32)
+        if embeddings.ndim == 1:
+            embeddings = embeddings.reshape(1, -1)
+        if embeddings.ndim != 2 or embeddings.shape[1] != self.index.d or len(ids) != embeddings.shape[0]:
+            raise ValueError(f"expected [len(ids) = {len(ids)}, {self.index.d}] embeddings, got {embeddings.shape}")
+        last = {item_id: i for i, item_id in enumerate(ids)}
+        pos = sorted(last.values())
+        rows, src, tail = [], [], []
+        for i in pos:
+            item_id = ids[i]
+            row = self.reverse_id_map.get(item_id)
+            if row is None:
+                if not self._free:
+                    tail.append(i)
+                    continue
+                row = heapq.heappop(self._free)
+                self.id_map[row] = item_id
+                self.reverse_id_map[item_id] = row
+                self._set_name(row, item_id)
+            rows.append(row)
+            src.append(i)
+        normalize = self.metric == "cosine"
+        if rows:
+            self.index.update_rows(np.asarray(rows, dtype=np.int64), embeddings[src], normalize=normalize)
+        if tail:
+            base = self.index.ntotal
+            self.index.add(embeddings[tail], normalize=normalize)
+            for j, i in enumerate(tail):
+                self.id_map[base + j] = ids[i]
+                self.reverse_id_map[ids[i]] = base + j
+            self._id_array = None
+        self.current_size = len(self.reverse_id_map)
+        logger.info("Upserted %d items (%d overwritten or reusing slots, %d appended). Live size: %d",
+                    len(pos), len(rows), len(tail), self.current_size)
+
+    def _drop_unmapped_rows(self) -> None:
+        """"in_place" after build / load: rows no id maps to (an id given twice keeps its last row) are removed."""
+        self.id_map = {row: item_id for item_id, row in sorted(self.reverse_id_map.items(), key=lambda t: t[1])}
+        self._id_array = None
+        dead = np.setdiff1d(np.arange(self.index.ntotal, dtype=np.int64),
+                            np.fromiter(self.id_map.keys(), dtype=np.int64, count=len(self.id_map)))
+        if dead.size:
+            self.index.remove_rows(dead)
+            self._free = dead.tolist()
+            heapq.heapify(self._free)
+        self.current_size = len(self.reverse_id_map)
+
+    def compact(self) -> np.ndarray:
+        """Drop removed slots on the device and renumber the id maps; returns the old -> new row map (-1 = removed)."""
+        if self.index is None:
+            raise ValueError("Index not built yet")
+        remap = self.index.compact()
+        self.id_map = {int(remap[r]): item_id for r, item_id in self.id_map.items() if remap[r] >= 0}
+        self.reverse_id_map = {item_id: r for r, item_id in self.id_map.items()}
+        self.current_size = len(self.reverse_id_map)
+        self._free = []
+        self._id_array = None
+        return remap
 
     def save(self, path: str):
-        """`<path>.faiss` = faiss' IndexFlatIP file, `<path>.pkl` = the id maps (reference retrieval.py:248-270)."""
+        """`<path>.faiss` = faiss' IndexFlatIP file, `<path>.pkl` = the id maps (reference retrieval.py:248-270).  Under
+        "in_place" the live rows are written renumbered densely (no tombstones: a faiss reader gets a plain IndexFlatIP)
+        with id maps to match."""
         if self.index is None:
             raise ValueError("No index to save")
         path = Path(path)
         path.parent.mkdir(parents=True, exist_ok=True)
-        write_ixfi(path.with_suffix(".faiss"), self.index.reconstruct_n(0, self.index.ntotal))
+        id_map, reverse_id_map, rows = self.id_map, self.reverse_id_map, self.index.reconstruct_n(0, self.index.ntotal)
+        if self.updates == "in_place":
+            live = np.asarray(sorted(self.id_map), dtype=np.int64)
+            rows = rows[live]
+            id_map = {j: self.id_map[int(r)] for j, r in enumerate(live)}
+            reverse_id_map = {item_id: j for j, item_id in id_map.items()}
+        write_ixfi(path.with_suffix(".faiss"), rows)
         with open(path.with_suffix(".pkl"), "wb") as f:
-            pickle.dump({"id_map": self.id_map, "reverse_id_map": self.reverse_id_map,
-                         "current_size": self.current_size, "config": self.config}, f)
+            pickle.dump({"id_map": id_map, "reverse_id_map": reverse_id_map,
+                         "current_size": len(reverse_id_map) if self.updates == "in_place" else self.current_size,
+                         "config": self.config}, f)
         logger.info("Saved index to %s", path)
 
     def load(self, path: str):
@@ -597,6 +916,9 @@ class B200FlatIndex(IndexBase):
         self.dimension = rows.shape[1]
         self.index = FlatIPDeviceIndex(self.dimension, storage=self.storage)
         self.index.add(rows, normalize=False)
+        self._free = []
+        if self.updates == "in_place":
+            self._drop_unmapped_rows()
         logger.info("Loaded index from %s with %d items", path, self.current_size)
 
 
