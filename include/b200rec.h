@@ -145,7 +145,10 @@ int b200rec_topk_sample_fanout(const void* catalogue, int64_t N, int64_t ld, con
  * b200rec_flat_ip_topk_filtered_fanout: the local top-k of a row shard starting from tau_init (nullable), stored to the
  * n_dst destinations.  Exactly one of allow_bits (bitmap path; ids = row + row_offset) and remap_rows (compacted
  * catalogue path: N = n_remap compacted rows, row j is local row remap_rows[j], ids = remap_rows[j] + row_offset, mapped
- * inside the select kernel) is given.  No allowed row (N == 0 or allow_n == 0): -FLT_MAX / -1 rows everywhere. */
+ * inside the select kernel) is given.  No allowed row (N == 0 or allow_n == 0): -FLT_MAX / -1 rows everywhere.
+ * b200rec_flat_ip_topk_masked_fanout: the same step with allow_bits and remap_rows each optional, so both may be given
+ * together: a compacted catalogue whose rows are tested against a bitmap over the compacted rows (a compact-path row
+ * filter on a shard with removed rows: the filter's compact live bits, allow_n = N).  Padding as above. */
 int b200rec_topk_sample_filtered(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q, int k,
                                  int k_out, int shards, const uint32_t* allow_bits, int64_t allow_n, float* out_vals,
                                  void* workspace, size_t workspace_bytes, void* stream);
@@ -158,6 +161,11 @@ int b200rec_flat_ip_topk_filtered_fanout(const void* catalogue, int64_t N, int64
                                          const int64_t* remap_rows, int64_t n_remap, const float* tau_init, int n_dst,
                                          void* const* dst_scores, void* const* dst_ids, void* workspace,
                                          size_t workspace_bytes, void* stream);
+int b200rec_flat_ip_topk_masked_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries, int64_t Q,
+                                       int k, int64_t row_offset, const uint32_t* allow_bits, int64_t allow_n,
+                                       const int64_t* remap_rows, int64_t n_remap, const float* tau_init, int n_dst,
+                                       void* const* dst_scores, void* const* dst_ids, void* workspace,
+                                       size_t workspace_bytes, void* stream);
 /* k-way merge of `parts` candidate lists [parts][Q][k_in] (id < 0 = empty, ids < 2^32) into the global top k_out under
  * the same order: the exchange step after the all-gather of per-GPU results.  *_part_stride = element distance
  * between consecutive parts (0 = dense, Q*k_in); non-dense strides let one all-gather carry scores and ids together. */

@@ -47,6 +47,8 @@ SIGNATURES = {
     "b200rec_topk_sample_filtered_fanout": (_I, [_P, _I64, _I64, _P, _I64, _I, _I, _I, _P, _I64, _I, _P, _P, _SZ, _P]),
     "b200rec_flat_ip_topk_filtered_fanout": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _I64, _P, _I64, _P, _I, _P, _P,
                                                   _P, _SZ, _P]),
+    "b200rec_flat_ip_topk_masked_fanout": (_I, [_P, _I64, _I64, _P, _I64, _I, _I64, _P, _I64, _P, _I64, _P, _I, _P, _P,
+                                                _P, _SZ, _P]),
     "b200rec_topk_merge": (_I, [_P, _P, _I, _I64, _I, _I, _I64, _I64, _P, _P, _P]),
     "b200rec_rescore_fp32": (_I, [_P, _I64, _P, _I64, _I64, _I64, _I, _P, _I64, _I, _P, _P]),
     "b200rec_mlp_forward": (_I, [_P, _I64, _P, _P, _I64, _P, _I64, _I, _I, _I, _P, _I64, _I, _P, _I, _P, _P]),

@@ -1686,6 +1686,27 @@ extern "C" int b200rec_topk_sample_filtered_fanout(const void* catalogue, int64_
                          workspace_bytes, stream);
 }
 
+// row-shard search step over an allow bitmap and / or a compacted catalogue with its remap table, from tau_init, stored
+// to every destination of the fan; `what` names the entry point in its error messages
+static int search_shard_fanout(const char* what, const void* catalogue, int64_t N, int64_t ld, const void* queries,
+                               int64_t Q, int k, int64_t row_offset, const uint32_t* allow_bits, int64_t allow_n,
+                               const int64_t* remap_rows, int64_t n_remap, const float* tau_init, int n_dst,
+                               void* const* dst_scores, void* const* dst_ids, void* workspace, size_t workspace_bytes,
+                               void* stream) {
+  using namespace b200;
+  OutFan fan;
+  if (make_fan(fan, n_dst, dst_scores, dst_ids, true)) return 1;
+  if (Q < 1) return fail("%s: Q must be >= 1", what);
+  if (k < 1 || k > 2048) return fail("%s: k must be in [1, 2048] (got %d)", what, k);
+  if (N < 0 || allow_n < 0) return fail("%s: N and allow_n must be >= 0", what);
+  if (remap_rows != nullptr && n_remap != N) return fail("%s: n_remap must equal N (one row per compacted row)", what);
+  const int64_t an = allow_bits != nullptr ? (allow_n < N ? allow_n : N) : N;
+  if (N == 0 || an == 0) return fan_fill(fan, Q * k, -FLT_MAX, -1, stream);
+  if (!catalogue || !workspace) return fail("%s: null catalogue or workspace", what);
+  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, allow_bits, an, tau_init, fan.s[0],
+                       fan.i[0], nullptr, k, 1, &fan, remap_rows, workspace, workspace_bytes, stream);
+}
+
 extern "C" int b200rec_flat_ip_topk_filtered_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries,
                                                     int64_t Q, int k, int64_t row_offset, const uint32_t* allow_bits,
                                                     int64_t allow_n, const int64_t* remap_rows, int64_t n_remap,
@@ -1696,15 +1717,17 @@ extern "C" int b200rec_flat_ip_topk_filtered_fanout(const void* catalogue, int64
   if (!queries) return fail("topk_filtered_fanout: null pointer");
   if ((allow_bits == nullptr) == (remap_rows == nullptr))
     return fail("topk_filtered_fanout: exactly one of allow_bits and remap_rows must be given");
-  OutFan fan;
-  if (make_fan(fan, n_dst, dst_scores, dst_ids, true)) return 1;
-  if (Q < 1) return fail("topk_filtered_fanout: Q must be >= 1");
-  if (k < 1 || k > 2048) return fail("topk_filtered_fanout: k must be in [1, 2048] (got %d)", k);
-  if (N < 0 || allow_n < 0) return fail("topk_filtered_fanout: N and allow_n must be >= 0");
-  if (remap_rows != nullptr && n_remap != N) return fail("topk_filtered_fanout: n_remap must equal N (one row per compacted row)");
-  const int64_t an = allow_bits != nullptr ? (allow_n < N ? allow_n : N) : N;
-  if (N == 0 || an == 0) return fan_fill(fan, Q * k, -FLT_MAX, -1, stream);
-  if (!catalogue || !workspace) return fail("topk_filtered_fanout: null catalogue or workspace");
-  return topk_dispatch(catalogue, N, ld, queries, Q, k, row_offset, nullptr, nullptr, allow_bits, an, tau_init, fan.s[0],
-                       fan.i[0], nullptr, k, 1, &fan, remap_rows, workspace, workspace_bytes, stream);
+  return search_shard_fanout("topk_filtered_fanout", catalogue, N, ld, queries, Q, k, row_offset, allow_bits, allow_n,
+                             remap_rows, n_remap, tau_init, n_dst, dst_scores, dst_ids, workspace, workspace_bytes, stream);
+}
+
+extern "C" int b200rec_flat_ip_topk_masked_fanout(const void* catalogue, int64_t N, int64_t ld, const void* queries,
+                                                  int64_t Q, int k, int64_t row_offset, const uint32_t* allow_bits,
+                                                  int64_t allow_n, const int64_t* remap_rows, int64_t n_remap,
+                                                  const float* tau_init, int n_dst, void* const* dst_scores,
+                                                  void* const* dst_ids, void* workspace, size_t workspace_bytes,
+                                                  void* stream) {
+  if (!queries) return b200::fail("topk_masked_fanout: null pointer");
+  return search_shard_fanout("topk_masked_fanout", catalogue, N, ld, queries, Q, k, row_offset, allow_bits, allow_n,
+                             remap_rows, n_remap, tau_init, n_dst, dst_scores, dst_ids, workspace, workspace_bytes, stream);
 }

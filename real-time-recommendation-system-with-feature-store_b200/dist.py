@@ -45,6 +45,17 @@ def shard_filter_rows(lo: int, n: int, rows=None, mask=None) -> np.ndarray:
     return np.unique(r[(r >= 0) & (r < n)])
 
 
+def shard_update_rows(lo: int, n: int, rows: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+    """(local rows, value positions) of the shard that holds global rows [lo, lo + n), from an update of GLOBAL rows
+    `rows` (int64) with one value row per entry: duplicates are resolved over the whole list first (the last occurrence
+    wins), then the shard keeps its own rows, ascending, and value i of its update is value positions[i] of the caller."""
+    r = np.asarray(rows, dtype=np.int64).reshape(-1)
+    u, first_rev = np.unique(r[::-1], return_index=True)     # ascending distinct rows, last occurrence of each
+    pos = r.size - 1 - first_rev
+    mine = (u >= lo) & (u < lo + n)
+    return u[mine] - lo, pos[mine]
+
+
 class ShardedRowFilter:
     """This rank's part of a row filter over the GLOBAL rows of a ShardedFlatIndex (`ShardedFlatIndex.row_filter`):
     `local` is the filter of the local shard (a retrieval.RowFilter over its local rows), which the shard's filtered
@@ -132,6 +143,8 @@ class ShardedFlatIndex:
     Filtered search (`search(..., sel=ShardedRowFilter)`) calls local_search(q, k, tau, out, sel=local filter) and
     local_sample(q, k, k_out, shards, sel=local filter); the filtered sampler always returns [Q,k_out] (padding rows of
     -FLT_MAX, or anything <= every real score, where it has nothing to sample).
+    Live catalogue (from_device_index): `update_rows` / `remove_rows` / `compact` / `n_live` over GLOBAL rows; a shard
+    with removed rows samples and searches its live rows only and, like a filtered shard, always contributes a sample.
     """
 
     def __init__(self, local_search: Callable, merge: Callable, group=None, local_sample: Optional[Callable] = None):
@@ -147,25 +160,20 @@ class ShardedFlatIndex:
         self.peer_index = None         # set by from_device_index: the local FlatIPDeviceIndex
         self.use_peer_exchange = False # from_device_index(peer_exchange=True): fan-out stores over NVLink
         self._ids_cache = {}
+        self._shard_sizes: Optional[np.ndarray] = None   # rows of every shard: gathered on the first mutation
 
     @classmethod
     def from_device_index(cls, index, group=None, peer_exchange: bool = True) -> "ShardedFlatIndex":
         from . import kernels as K
 
         def local(q_op, k, tau=None, out=None, sel=None):
-            if sel is not None:
-                return index.search_filtered_shard(q_op, k, sel, tau, out=out)
-            return index.search_device(q_op, k, tau_init=tau, out=out)
+            return index.search_shard(q_op, k, tau, sel=sel, out=out)
 
         def merge(s, i, k):
             return K.topk_merge(s, i, k)
 
         def sample(q_op, k, k_out=None, shards=1, sel=None):
-            if sel is not None:
-                return index.sample_filtered(q_op, k, k if k_out is None else k_out, shards, sel)
-            if not index.has_sample_pass(q_op.shape[0], k):
-                return None
-            return index.sample_device(q_op, k, k_out, shards)
+            return index.sample_shard(q_op, k, k_out, shards, sel=sel)
 
         obj = cls(local, merge, group, sample)
         obj.packed_exchange = True
@@ -184,6 +192,89 @@ class ShardedFlatIndex:
         if ix.storage != "bf16":
             raise ValueError("row-sharded filtered search needs bf16 storage (the index of this shard stores fp32)")
         return ShardedRowFilter(ix.row_filter(rows=shard_filter_rows(ix.row_offset, ix.ntotal, rows, mask)))
+
+    # ------------------------------------------------------------------ live catalogue (GLOBAL rows)
+    def _local_index(self, what: str):
+        if self.peer_index is None:
+            raise RuntimeError(f"{what} needs a ShardedFlatIndex built by from_device_index")
+        return self.peer_index
+
+    def _all_gather(self, a: np.ndarray) -> np.ndarray:
+        """Small host array of every rank -> [world, *a.shape] (one collective; outside the search path)."""
+        world = dist.get_world_size(self.group)
+        dev = self.peer_index.device if dist.get_backend(self.group) == "nccl" else "cpu"
+        t = torch.from_numpy(np.ascontiguousarray(a).reshape(-1)).to(dev)
+        out = torch.empty((world * t.numel(),), dtype=t.dtype, device=dev)
+        dist.all_gather_into_tensor(out, t, group=self.group)
+        return out.cpu().numpy().reshape((world,) + a.shape)
+
+    def _global_rows(self, rows, what: str) -> np.ndarray:
+        """Global rows checked against the global row count, the same on every rank (ValueError before device work)."""
+        from .retrieval import check_rows
+        if self._shard_sizes is None:
+            self._shard_sizes = self._all_gather(np.array([self.peer_index.ntotal], np.int64))[:, 0]
+        return check_rows(rows, int(self._shard_sizes.sum()), what)
+
+    def update_rows(self, rows, x, normalize: bool = False) -> None:
+        """`FlatIPDeviceIndex.update_rows` over GLOBAL rows: x[i] (host or device [n, d]) goes to global row rows[i],
+        the last occurrence of a repeated row wins, a removed row is revived (how a new item takes a freed slot).  Every
+        rank passes the same arguments; each copies only its shard's slice of x to its device.  No collective (except
+        the one-time gather of the shard sizes); ValueError on every rank for rows outside [0, global ntotal), non-integer
+        rows or a shape mismatch, before any device work."""
+        ix = self._local_index("update_rows")
+        if _world()[0] == 1:
+            ix.update_rows(rows, x, normalize)
+            return
+        r = self._global_rows(rows, "update_rows")
+        xt = torch.as_tensor(x)
+        if xt.dim() != 2 or xt.shape[1] != ix.d or xt.shape[0] != r.size:
+            raise ValueError(f"update_rows: expected [{r.size}, {ix.d}] rows, got {tuple(xt.shape)}")
+        local, pos = shard_update_rows(ix.row_offset, ix.ntotal, r)
+        if local.size:
+            ix.update_rows(local, xt[torch.from_numpy(pos).to(xt.device)], normalize)
+
+    def remove_rows(self, rows) -> int:
+        """`FlatIPDeviceIndex.remove_rows` over GLOBAL rows; returns how many live rows were removed ON THIS SHARD.
+        Every rank passes the same rows; no collective (except the one-time gather of the shard sizes)."""
+        ix = self._local_index("remove_rows")
+        if _world()[0] == 1:
+            return ix.remove_rows(rows)
+        r = self._global_rows(rows, "remove_rows")
+        return ix.remove_rows(shard_filter_rows(ix.row_offset, ix.ntotal, rows=r))
+
+    def n_live(self) -> int:
+        """Live rows of the whole catalogue (one small collective: call it outside the search path)."""
+        ix = self._local_index("n_live")
+        if _world()[0] == 1:
+            return ix.n_live
+        return int(self._all_gather(np.array([ix.n_live], np.int64)).sum())
+
+    def compact(self) -> np.ndarray:
+        """Every shard drops its removed rows (rows never move between shards) and takes its new row_offset: returns the
+        GLOBAL old -> new row map (int64 [old global ntotal], -1 for removed rows), the same on every rank.  Row filters
+        built before are rejected afterwards; the per-shape exchange decisions are made again on the next search."""
+        ix = self._local_index("compact")
+        world = _world()[0]
+        local = ix.compact()
+        # a shard that shrank may have lost its sampling pass: the agreed ("use") and peer ("peer") choices are stale
+        for key in [key for key in self._ids_cache if key[0] in ("use", "peer")]:
+            del self._ids_cache[key]
+        if world == 1:
+            return local
+        sizes = self._all_gather(np.array([local.size, ix.ntotal], np.int64))     # rows before / after, every shard
+        old, new = sizes[:, 0], sizes[:, 1]
+        old_off = np.concatenate([[0], np.cumsum(old)[:-1]])
+        new_off = np.concatenate([[0], np.cumsum(new)[:-1]])
+        ix.row_offset = int(new_off[dist.get_rank(self.group)])
+        self._shard_sizes = new
+        keep = np.zeros(int(old.max()), np.uint8)
+        keep[: local.size] = local >= 0
+        keeps = self._all_gather(keep).astype(bool)
+        out = np.full(int(old.sum()), -1, np.int64)
+        for p in range(world):
+            kept = np.flatnonzero(keeps[p, : old[p]])
+            out[old_off[p] + kept] = new_off[p] + np.arange(kept.size, dtype=np.int64)
+        return out
 
     def _peer(self, q: int, k: int, world: int, device):
         """Peer gather buffers for this shape, or None when symmetric memory is unavailable / a shard has no sampling
@@ -208,17 +299,12 @@ class ShardedFlatIndex:
 
     def _search_peer(self, px: "_PeerExchange", queries, k: int, world: int, sel=None):
         ix = self.peer_index
-        if sel is None:
-            ix.sample_fanout(queries, k, px.tau_all.shape[2], world, px.tau_dst)  # (1) sample -> every gather buffer
-        else:                                           # allowed rows only; padding rows where there is nothing to sample
-            ix.sample_filtered(queries, k, px.tau_all.shape[2], world, sel, dst=px.tau_dst)
+        # (1) sample -> every gather buffer (live and allowed rows only; padding rows where there is nothing to sample)
+        ix.sample_shard(queries, k, px.tau_all.shape[2], world, sel=sel, dst=px.tau_dst)
         px.barrier(0)
         from . import kernels as K
         tau = K.topk_pooled_kth(px.tau_all, k)                                   # (2) k-th best of the pooled sample
-        if sel is None:
-            ix.search_fanout(queries, k, tau, px.s_dst, px.i_dst)                # (3) local top-k -> every gather buffer
-        else:
-            ix.search_filtered_shard(queries, k, sel, tau, dst=(px.s_dst, px.i_dst))
+        ix.search_shard(queries, k, tau, sel=sel, dst=(px.s_dst, px.i_dst))      # (3) local top-k -> every gather buffer
         px.barrier(1)
         return self.merge(px.s_all, px.i_all, k)                                 # (4) k-way select
 
@@ -277,6 +363,8 @@ class ShardedFlatIndex:
         lsel = None if sel is None else sel.local
         kw = {} if sel is None else {"sel": lsel}
         if world == 1:
+            if sel is None and self.peer_index is not None:   # the one-GPU search: live rows of either storage
+                return self.peer_index.search_device(queries, k)
             return self.local_search(queries, k, **kw)
         if self.peer_index is not None and self.use_peer_exchange:
             px = self._peer(int(queries.shape[0]), k, world, queries.device)

@@ -274,6 +274,25 @@ def flat_ip_topk_filtered_fanout(catalogue: Optional[torch.Tensor], queries: tor
             "flat_ip_topk_filtered_fanout")
 
 
+def flat_ip_topk_masked_fanout(catalogue: Optional[torch.Tensor], queries: torch.Tensor, k: int, row_offset: int,
+                               allow_bits: Optional[torch.Tensor], allow_n: int, remap_rows: Optional[torch.Tensor],
+                               tau_init: Optional[torch.Tensor], dst_scores, dst_ids,
+                               workspace: Optional[torch.Tensor]) -> None:
+    """flat_ip_topk_filtered_fanout with allow_bits and remap_rows each optional: both together search a compacted
+    catalogue whose rows are also tested against a bitmap over the compacted rows (allow_n of them)."""
+    assert allow_bits is None or allow_bits.dtype == torch.int32
+    assert remap_rows is None or (remap_rows.dtype == torch.int64 and catalogue is not None
+                                  and remap_rows.numel() == catalogue.shape[0])
+    n = 0 if catalogue is None else catalogue.shape[0]
+    n_remap = 0 if remap_rows is None else remap_rows.numel()
+    N.check(N.lib().b200rec_flat_ip_topk_masked_fanout(N.ptr(catalogue), n, queries.stride(0), N.ptr(queries),
+                                                       queries.shape[0], k, row_offset, N.ptr(allow_bits), allow_n,
+                                                       N.ptr(remap_rows), n_remap, N.ptr(tau_init), len(dst_scores),
+                                                       _ptr_table(dst_scores), _ptr_table(dst_ids), N.ptr(workspace),
+                                                       0 if workspace is None else workspace.numel(), N.stream()),
+            "flat_ip_topk_masked_fanout")
+
+
 def topk_has_sample(n: int, ld: int, q: int, k: int) -> bool:
     return bool(N.lib().b200rec_topk_has_sample(n, ld, q, k))
 

@@ -50,6 +50,22 @@ def check_dimension(d: int, storage: str) -> None:
     raise ValueError(msg)
 
 
+def check_rows(rows, ntotal: int, what: str) -> np.ndarray:
+    """Host validation of a row list (before anything reaches the device): 1-D integers in [0, ntotal), as int64."""
+    r = np.asarray(rows.detach().cpu() if torch.is_tensor(rows) else rows)
+    if r.ndim != 1:
+        raise ValueError(f"{what}: rows must be a 1-D integer array (got shape {r.shape})")
+    if r.size == 0:
+        return np.zeros(0, dtype=np.int64)
+    if not np.issubdtype(r.dtype, np.integer):
+        raise ValueError(f"{what}: rows must be an integer array (got {r.dtype})")
+    r = r.astype(np.int64, copy=False)
+    bad = (r < 0) | (r >= ntotal)
+    if bad.any():
+        raise ValueError(f"{what}: row {int(r[bad][0])} is outside [0, ntotal = {ntotal})")
+    return r
+
+
 class IndexBase(ABC):
     """Abstract base class for ANN indices (reference retrieval.py:16-46)."""
 
@@ -147,9 +163,9 @@ class FlatIPDeviceIndex:
     exactly the unmutated code; after it, a live-row bitmap (one bit per slot, kept on the device and mirrored on the
     host) is tested inside the fused kernel.  Mutations are enqueued on the caller's current CUDA stream: a search issued
     on that stream after a mutation call has returned sees the mutation (`search` / `search_stream` search on the current
-    stream, so batches submitted after an update see it).  The row-sharded steps (`sample_device`, `sample_fanout`,
+    stream, so batches submitted after an update see it).  The older row-shard steps (`sample_device`, `sample_fanout`,
     `search_fanout`, `sample_filtered`, `search_filtered_shard`) do not read the live bitmap and refuse an index with
-    removed rows.
+    removed rows; `sample_shard` / `search_shard`, which `dist.ShardedFlatIndex` runs, read it.
     """
 
     @staticmethod
@@ -251,19 +267,7 @@ class FlatIPDeviceIndex:
         return self.ntotal - self._n_dead
 
     def _check_rows(self, rows, what: str) -> np.ndarray:
-        """Host validation of a row list (before anything reaches the device): 1-D integers in [0, ntotal)."""
-        r = np.asarray(rows.detach().cpu() if torch.is_tensor(rows) else rows)
-        if r.ndim != 1:
-            raise ValueError(f"{what}: rows must be a 1-D integer array (got shape {r.shape})")
-        if r.size == 0:
-            return np.zeros(0, dtype=np.int64)
-        if not np.issubdtype(r.dtype, np.integer):
-            raise ValueError(f"{what}: rows must be an integer array (got {r.dtype})")
-        r = r.astype(np.int64, copy=False)
-        bad = (r < 0) | (r >= self.ntotal)
-        if bad.any():
-            raise ValueError(f"{what}: row {int(r[bad][0])} is outside [0, ntotal = {self.ntotal})")
-        return r
+        return check_rows(rows, self.ntotal, what)
 
     def _ensure_live(self) -> None:
         if self._live_bits is None:
@@ -474,6 +478,71 @@ class FlatIPDeviceIndex:
                                             torch.empty((nq, k), dtype=torch.int64, device=self.device))
         K.flat_ip_topk_filtered_fanout(cat, q_op, k, self.row_offset, bits, allow_n, remap, tau, [d.data_ptr()],
                                        [i.data_ptr()], ws)
+        return d, i
+
+    # ------------------------------------------------------------------ live-aware row-shard steps (dist.ShardedFlatIndex)
+    def _live_operand(self, sel: Optional[RowFilter]):
+        """(catalogue, allow_bits, allow_n, remap_rows) a row-shard step runs over on an index with removed rows: the
+        live bits over the local catalogue, a bitmap filter ANDed with them, or a compacted filter's rows with its
+        compact-row live bits and its local row list.  No live row: (None, None, 0, None), answered with padding."""
+        if self.storage != "bf16":
+            raise ValueError("row-sharded search over an index with removed rows needs bf16 storage (an fp32-storage "
+                             "shard re-scores its candidates from fp32 rows, which the sharded exchange does not carry)")
+        if sel is None:
+            if self.n_live == 0:
+                return None, None, 0, None
+            return self._cat[: self.ntotal], self._live_bits, self.ntotal, None
+        cat, bits, allow_n, remap = self._shard_operand(sel, None)
+        if cat is None:
+            return None, None, 0, None
+        if remap is None:
+            return cat, sel.live_bits(), allow_n, None
+        return cat, sel._compact_bits, sel.n_allowed, remap
+
+    def sample_shard(self, q_op: torch.Tensor, k: int, k_out: Optional[int] = None, shards: int = 1,
+                     sel: Optional[RowFilter] = None, dst=None) -> Optional[torch.Tensor]:
+        """Sampling step of a row-sharded search over the live (and, with `sel`, allowed) rows: the k_out (default k)
+        best group maxima per query [nq, k_out], or stored to every address in `dst`.  An index with no removed row runs
+        exactly sample_device / sample_fanout / sample_filtered (unfiltered: None when the shape has no sampling pass);
+        one with removed rows runs the masked sampling pass and always answers, with -FLT_MAX rows where it has nothing
+        to sample, so a shard's removals never change what the other shards do."""
+        k_out = k if k_out is None else k_out
+        if self._n_dead == 0:
+            if sel is not None:
+                return self.sample_filtered(q_op, k, k_out, shards, sel, dst=dst)
+            if dst is not None:
+                self.sample_fanout(q_op, k, k_out, shards, dst)
+                return None
+            if not self.has_sample_pass(q_op.shape[0], k):
+                return None
+            return self.sample_device(q_op, k, k_out, shards)
+        cat, bits, allow_n, _ = self._live_operand(sel)
+        ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
+        return K.topk_sample_filtered(cat, q_op, k, k_out, shards, bits, allow_n, ws, dst)
+
+    def search_shard(self, q_op: torch.Tensor, k: int, tau, sel: Optional[RowFilter] = None, out=None, dst=None):
+        """Local exact top-k of a row-sharded search over the live (and, with `sel`, allowed) rows from the pooled
+        threshold `tau` ([nq] or None), global row ids, -1 / -FLT_MAX padding.  Returns (D, I) (written into `out` when
+        given), or stores the rows to every (dst[0][d], dst[1][d]) address and returns None.  An index with no removed
+        row runs exactly search_device(tau_init=) / search_fanout / search_filtered_shard; one with removed rows runs one
+        fused search that tests the live bits (and the filter) and maps compacted ids back, bf16 storage only."""
+        if self._n_dead == 0:
+            if sel is not None:
+                return self.search_filtered_shard(q_op, k, sel, tau, out=out, dst=dst)
+            if dst is not None:
+                self.search_fanout(q_op, k, tau, dst[0], dst[1])
+                return None
+            return self.search_device(q_op, k, tau_init=tau, out=out)
+        cat, bits, allow_n, remap = self._live_operand(sel)
+        ws = None if cat is None else self._workspace(q_op.shape[0], k, cat.shape[0])
+        if dst is not None:
+            K.flat_ip_topk_masked_fanout(cat, q_op, k, self.row_offset, bits, allow_n, remap, tau, dst[0], dst[1], ws)
+            return None
+        nq = q_op.shape[0]
+        d, i = out if out is not None else (torch.empty((nq, k), dtype=torch.float32, device=self.device),
+                                            torch.empty((nq, k), dtype=torch.int64, device=self.device))
+        K.flat_ip_topk_masked_fanout(cat, q_op, k, self.row_offset, bits, allow_n, remap, tau, [d.data_ptr()],
+                                     [i.data_ptr()], ws)
         return d, i
 
     def search_device(self, q_op: torch.Tensor, k: int, exclude_indptr=None, exclude_rows=None, tau_init=None,
